@@ -3,6 +3,10 @@
 
     python bench.py --gpus N --steps K --warmup W                     # the CUDA path (this repo)
     python bench.py --impl reference --gpus N --steps K --warmup W    # the reference's CPU algorithm
+    python bench.py ... --dump-outputs DIR     # also write the last timed step's results as DIR/*.npy
+
+The inputs are a function of the arguments alone (seeded), so two builds run with the same arguments can be
+compared output for output.  Nothing is written under the repository: the tree may be read-only.
 
 One "step" = one batch of queries searched through the whole path (centroid scoring -> probe -> candidates ->
 approximate score -> cut -> decompress + MaxSim -> top-k) against a synthetic index resident in HBM.
@@ -46,6 +50,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True     # no __pycache__ in the tree
 if "--impl" in sys.argv and "reference" in sys.argv:
     # torchrun exports OMP_NUM_THREADS=1; the reference arm is a CPU measurement and uses every host thread
     os.environ["OMP_NUM_THREADS"] = str(os.cpu_count() or 1)
@@ -85,7 +90,11 @@ def parse_args():
     ap.add_argument("--pool", type=int, default=256, help="centroids per topic pool")
     ap.add_argument("--res-sigma", type=float, default=0.05, help="per-dimension residual scale")
     ap.add_argument("--query-noise", type=float, default=0.15)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's results as DIR/passage_ids.npy, scores.npy, counts.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     world = int(os.environ.get("WORLD_SIZE", 1))
     if a.docs_total <= 0:
         a.docs_total = 1_000_000 if world == 1 else 10_000_000
@@ -310,6 +319,29 @@ def workload_config(args, world):
             "l2": "index (>= 20 GB/GPU) exceeds the 126 MB L2; a distinct query batch every step"}
 
 
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(path, ids, scores, counts):
+    """Write what one search call returned, one row per query, so that two builds can be compared output for output:
+    passage_ids.npy (f64, exact for any doc id below 2^53), scores.npy (f32) and counts.npy (f64).  Slots past a row's
+    count are undefined in the library's output; they are written as id -1 and score 0.  When the arrays exceed 64 MB,
+    a fixed, seeded sample of rows is written instead, with the sampled row numbers in rows.npy."""
+    ids, scores, counts = np.asarray(ids, np.int64), np.asarray(scores, np.float32), np.asarray(counts, np.int64)
+    valid = np.arange(ids.shape[1])[None, :] < counts[:, None]
+    out = {"passage_ids": np.where(valid, ids, -1).astype(np.float64),
+           "scores": np.where(valid, scores, np.float32(0)).astype(np.float32),
+           "counts": counts.astype(np.float64)}
+    row_bytes = sum(a[0].nbytes for a in out.values()) + 8
+    if len(counts) * row_bytes > DUMP_MAX_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(len(counts), DUMP_MAX_BYTES // row_bytes, replace=False))
+        out = {name: a[rows] for name, a in out.items()}
+        out["rows"] = rows.astype(np.float64)
+    os.makedirs(path, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def same_results(a, b):
     ids = sum(int(x.passage_ids.tolist() == y.passage_ids.tolist()) for x, y in zip(a, b))
     dmax = 0.0
@@ -422,6 +454,8 @@ def run_b200(args):
         return stage_ms, kern_ms, work, launches, dev_ms, 1e3 * (time.perf_counter() - tw)
 
     stage_ms, kern_ms, work, launches, dev_ms, wall_ms = timed_region()
+    if args.dump_outputs and rank == 0:      # every rank holds the same merged results
+        dump_outputs(args.dump_outputs, d_ids.cpu().numpy(), d_sc.cpu().numpy(), d_cn.cpu().numpy())
     # the same steps with the batch searched as one slice (pb_set_lanes(1)): kernels run alone, so these are the
     # per-kernel times that are not stretched by a co-running slice
     one_lane = None
@@ -678,9 +712,14 @@ def run_reference(args):
             oracle.search_sharded(shards, bases, q, po)
     t0 = time.perf_counter()
     for i in range(args.steps):
-        for q in step_q(args.warmup + i):
-            oracle.search_sharded(shards, bases, q, po)
+        last = [oracle.search_sharded(shards, bases, q, po) for q in step_q(args.warmup + i)]
     s = time.perf_counter() - t0
+    if args.dump_outputs:
+        ids = np.full((len(last), args.top_k), -1, np.int64)
+        sc = np.zeros((len(last), args.top_k), np.float32)
+        for r, res in enumerate(last):
+            ids[r, :len(res.passage_ids)], sc[r, :len(res.scores)] = res.passage_ids, res.scores
+        dump_outputs(args.dump_outputs, ids, sc, [len(res.passage_ids) for res in last])
     qps = per_step * args.steps / s
     cores = oracle.lib().po_num_threads()
     sample = (f"{per_step} queries per step (the first of each {args.batch}-query batch of the b200 arm), {args.steps} steps; "

@@ -2,6 +2,7 @@
 from __future__ import annotations
 
 import os
+import shutil
 import subprocess
 import sys
 
@@ -18,6 +19,19 @@ NVCC_FLAGS = [
 ]
 
 
+def cuda_tool(name: str) -> str:
+    """A CUDA toolkit program: from PATH, else from $CUDA_HOME/bin (default /usr/local/cuda), where the toolkit
+    installs it even when a user's PATH does not name that directory."""
+    found = shutil.which(name)
+    if found:
+        return found
+    home = os.environ.get("CUDA_HOME") or os.environ.get("CUDA_PATH") or "/usr/local/cuda"
+    path = os.path.join(home, "bin", name)
+    if not os.access(path, os.X_OK):
+        raise RuntimeError(f"{name} is neither on PATH nor in {os.path.dirname(path)}; set CUDA_HOME")
+    return path
+
+
 def needs_build() -> bool:
     if not os.path.exists(LIB):
         return True
@@ -28,7 +42,7 @@ def needs_build() -> bool:
 def build_library(force: bool = False, verbose: bool = False) -> str:
     if not force and not needs_build():
         return LIB
-    nvcc = os.environ.get("NVCC", "nvcc")
+    nvcc = os.environ.get("NVCC") or cuda_tool("nvcc")
     cmd = [nvcc] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + \
           [os.path.join(CSRC, s) for s in SOURCES] + ["-o", LIB]
     env = dict(os.environ)

@@ -28,7 +28,9 @@ def test_header_symbols_all_exported(npb):
 
 def test_library_targets_sm100a_only(npb):
     import subprocess
-    out = subprocess.run(["cuobjdump", "-lelf", npb.LIB_PATH], capture_output=True, text=True).stdout
+    from importlib import import_module
+    cuobjdump = import_module("next_plaid_b200.build").cuda_tool("cuobjdump")
+    out = subprocess.run([cuobjdump, "-lelf", npb.LIB_PATH], capture_output=True, text=True).stdout
     assert "sm_100a" in out
     assert not re.search(r"sm_(?!100a)\d+", out), out
 
