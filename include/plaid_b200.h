@@ -379,9 +379,12 @@ PB_API pb_status pb_create_index(const float *embeddings, const int64_t *doc_len
  * One process per GPU; shard g holds a contiguous doc-id range (pb_index_desc.doc_id_base) with the
  * centroids replicated.  After pb_index_comm_init every pb_search_batch on the handle is a collective:
  * all ranks call it with the same queries and parameters and all receive the same global result,
- * bit-identical to searching the unsharded index.  Two NCCL all-gathers per sub-batch (per-shard
- * top-M approximate keys, then exact triples) reproduce the reference's GLOBAL n_full_scores/4 cut
- * (search.rs:460-469) and its stable final sort (search.rs:496).
+ * bit-identical to searching the unsharded index.  Per sub-batch, an all-gather of the per-shard top-M
+ * approximate keys and two of the exact (key, rank) and (id, score) words reproduce the reference's GLOBAL
+ * n_full_scores/4 cut (search.rs:460-469) and its stable final sort (search.rs:496).  A fourth
+ * all-gather of one 8-byte flag word per rank comes first, so that all ranks redo a sub-batch on the
+ * exact path together when any shard's tensor-core pass gives up; and once per call the ranks
+ * all-gather their sub-batch sizes and all use the smallest.
  */
 PB_API pb_status pb_comm_unique_id(uint8_t *out128);   /* rank 0: 128-byte NCCL unique id */
 PB_API pb_status pb_index_comm_init(pb_index *ix, const uint8_t *id128, int32_t rank, int32_t world);

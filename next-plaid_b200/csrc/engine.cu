@@ -243,8 +243,8 @@ struct Workspace {
     cudaEvent_t call_ev[2] = {};                // around a whole search call
     DevBuf Q, qoff, ST, partial, sel, cells, ncells, bitmap, cand, ncand, approx, keys, kept, nkept, tokp, maxkey,
         exact, fkeys, oids, oscores, ocounts, subset, subset_bits, elig, misc, list, counters, lkeys, ST16, qrange, qflag, lsum, cand2, ncand2,  cellbits,
-        gkeys, krank, payload, gfkeys, gpayload, cmax16, tau16, plist, pcount, Qi, Qh16t, Ql16t, ST16b, k1diag, k1rows, ulist, nulist, est, kept2, krank2, nkept2, tokp2, ktok2, qnmax, qexp, qrange_tc, mslot, slicecnt, rcmax, rcpairs, rcn, cellflags, estkey, srcrank, xpairs, xnpairs, needexact, gbase;
-    HostBuf hq, hres, hcounts;
+        gkeys, krank, payload, gfkeys, gpayload, cmax16, tau16, plist, pcount, Qi, Qh16t, Ql16t, ST16b, k1diag, k1rows, ulist, nulist, est, kept2, krank2, nkept2, tokp2, ktok2, qnmax, qexp, qrange_tc, mslot, slicecnt, rcmax, rcpairs, rcn, cellflags, estkey, srcrank, xpairs, xnpairs, needexact, gbase, redoflag;
+    HostBuf hq, hres, hcounts, hredo;
     pb_status init() {
         CK(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
         for (auto &e : ev) CK(cudaEventCreate(&e));
@@ -991,6 +991,24 @@ static pb_status shard_allgather(pb_index *ix, cudaStream_t stream, const void *
     return PB_OK;
 }
 
+// A collective decision of a sharded handle: one 64-bit word per rank, all-gathered, read on every rank's host
+// (returned in ws.hredo[0 .. world)).  `d_lo`, when given, is a device int copied over the low half of `mine` (a flag
+// raised on the device).
+static pb_status shard_vote(pb_index *ix, Workspace &ws, u64 mine, const int *d_lo, const u64 **all) {
+    const int G = ix->world;
+    CKS(ws.redoflag.ensure((size_t)(G + 1) * 8));
+    CKS(ws.hredo.ensure((size_t)(G + 1) * 8));
+    u64 *h = ws.hredo.as<u64>();
+    h[G] = mine;
+    CK(cudaMemcpyAsync(ws.redoflag.p, h + G, 8, cudaMemcpyHostToDevice, ws.stream));
+    if (d_lo) CK(cudaMemcpyAsync(ws.redoflag.p, d_lo, 4, cudaMemcpyDeviceToDevice, ws.stream));
+    CKS(shard_allgather(ix, ws.stream, ws.redoflag.p, ws.redoflag.as<u64>() + 1, 1));
+    CK(cudaMemcpyAsync(h, ws.redoflag.as<u64>() + 1, (size_t)G * 8, cudaMemcpyDeviceToHost, ws.stream));
+    CK(cudaStreamSynchronize(ws.stream));
+    *all = h;
+    return PB_OK;
+}
+
 struct KeptView {  // the docs the exact stage scores: the cut's output, or the filter's survivors
     uint32_t *kept;
     int *nkept;
@@ -1313,11 +1331,28 @@ static pb_status search_impl_inner(pb_index *ix, const pb_search_params *p, cons
     size_t per_q = (size_t)ix->K * QS_all * sizeof(float);
     if (per_q >= ((size_t)1 << 32))
         return pb_fail(PB_ERR_UNSUPPORTED, "num_centroids x query tokens x 4 = %zu bytes per query exceeds 2^32", per_q);
-    // sub-batch size: the score tables (16-bit always, fp32 only on the exact path) and the per-(query, doc) scratch
-    // (candidate lists, code sums, approximate scores, cut keys, bitmap: 24.2 bytes per document) share one budget
-    const size_t per_q_all = (size_t)ix->K * QS_all * (k1_tc_usable(ix) ? 2 : 6) + (size_t)ix->D * 24 + (size_t)ix->D / 8 + 4096;
+    // the score table comes from the tensor cores unless something needs the dense fp32 S (an eligibility filter,
+    // the radix-select probe, a trace) or the shape is outside the kernel's (DESIGN.md "a2"); all of that is fixed for
+    // the call except the sub-batch's row width QS / 8 <= 32
+    const bool fast = ix->fast_approx && !io.trace;  // trace wants every candidate's exact approximate score
+    int n_chunks_k = 0;
+    probe_chunk_rows(ix->K, n_probe, &n_chunks_k);
+    const bool tc_call = k1_tc_usable(ix) && fast && ix->probe16 && !ix->k1_diag && !all_eligible && !big_probe && !d_elig &&
+                         n_chunks_k >= n_probe && n_probe <= 192;
+    // sub-batch size: the score tables (16-bit on the tensor-core path; fp32 and 16-bit otherwise) and the per-(query,
+    // doc) scratch (candidate lists, code sums, approximate scores, cut keys, bitmap: 24.2 bytes per document) share
+    // one budget
+    const bool tc_all = tc_call && QS_all / 8 <= 32;  // every sub-batch of the call can take the tensor-core path
+    const size_t per_q_all = (size_t)ix->K * QS_all * (tc_all ? 2 : 6) + (size_t)ix->D * 24 + (size_t)ix->D / 8 + 4096;
     int QB = (int)std::max<size_t>(1, std::min<size_t>((size_t)Bt, ix->st_budget / std::max(g_budget_div, 1) / per_q_all));
     QB = std::min(QB, 256);
+    if (sharded) {
+        // every rank must cut the call into the same sub-batches (each sub-batch is a set of exchanges), but per_q_all
+        // depends on the shard's own documents and tensor-core operands: the group takes the smallest size
+        const u64 *all = nullptr;
+        CKS(shard_vote(ix, ws, (u64)QB, nullptr, &all));
+        for (int g = 0; g < ix->world; ++g) QB = std::min<int>(QB, (int)all[g]);
+    }
     QB = (int)((Bt + (Bt + QB - 1) / QB - 1) / ((Bt + QB - 1) / QB));  // equal sub-batches
 
     const bool prof = ix->profiling;
@@ -1332,16 +1367,13 @@ static pb_status search_impl_inner(pb_index *ix, const pb_search_params *p, cons
         for (int b = 0; b < B; ++b) nq_max = std::max(nq_max, qoff[b + 1] - qoff[b]);
         const int QS = query_row_tokens(nq_max);
         int *L = g_stats.launches;
-        const bool fast = ix->fast_approx && !io.trace;  // trace wants every candidate's exact approx score
-        // the score table comes from the tensor cores unless something needs the dense fp32 S (an eligibility filter,
-        // the radix-select probe, a trace) or the shape is outside the kernel's (DESIGN.md "a2")
-        int n_chunks_k = 0;
-        probe_chunk_rows(ix->K, n_probe, &n_chunks_k);
-        const bool want_tc = k1_tc_usable(ix) && fast && ix->probe16 && !ix->k1_diag && !all_eligible && !big_probe && !d_elig &&
-                             QS / 8 <= 32 && n_chunks_k >= n_probe && n_probe <= 192;
-        // One pass over the sub-batch.  use_tc: a flagged query or a probe-list overflow raises a device flag instead of
-        // being read back mid-way; the pass then finishes on (memory-safe) garbage and *redo asks for the exact pass.
-        auto run_sub = [&](const bool use_tc, bool *redo) -> pb_status {
+        const bool want_tc = tc_call && QS / 8 <= 32;
+        // One pass over the sub-batch.  use_tc: a flagged query, a probe-list overflow or a re-check overflow raises a
+        // device flag instead of being read back mid-way; the pass then finishes on (memory-safe) garbage and *redo asks
+        // for the exact pass.  vote (a sharded handle's first pass over the sub-batch, on every rank whatever path it
+        // takes): the ranks' flags are gathered before the first exchange, so that every rank abandons the pass
+        // together and the ranks' exchanges stay paired.
+        auto run_sub = [&](const bool use_tc, const bool vote, bool *redo) -> pb_status {
         *redo = false;
         if (prof) CK(cudaEventRecord(ws.ev[0], ws.stream));
         // ---- H2D ----
@@ -1550,6 +1582,22 @@ static pb_status search_impl_inner(pb_index *ix, const pb_search_params *p, cons
         CK(cudaGetLastError());
         L[PB_STAGE_APPROX] += 1;
         if (prof) CK(cudaEventRecord(ws.ev[5], ws.stream));
+        if (vote) {
+            // The probe flags are the same on every rank (a2/a3 are replicated), a re-check overflow is not: it depends
+            // on this shard's documents.  Nor is the path: a rank without tensor-core operands (a shard with no tokens)
+            // or with other settings runs the exact pass and votes 0.  Every rank's flag word is gathered here, before
+            // exchange 1, and the pass is abandoned on all ranks if any rank raised it; a lone redo would pair its
+            // exchanges with the peers' next ones.  The kernels so far have restored their scratch invariants
+            // (bitmaps, re-check maxima).
+            const u64 *all = nullptr;
+            CKS(shard_vote(ix, ws, 0, tc ? d_probe_fallback : nullptr, &all));
+            u64 any = 0;
+            for (int g = 0; g < ix->world; ++g) any |= all[g];
+            if (any) {
+                *redo = true;
+                return PB_OK;
+            }
+        }
 
         // ---- a6 cut ----
         CKS(ws.kept.ensure((size_t)B * Mcap * 4));
@@ -1836,10 +1884,10 @@ static pb_status search_impl_inner(pb_index *ix, const pb_search_params *p, cons
         return PB_OK;
         };  // run_sub
         bool redo = false;
-        CKS(run_sub(want_tc, &redo));
+        CKS(run_sub(want_tc, sharded, &redo));
         if (redo) {
             g_stats.work.n_k1_tc_redo += 1;
-            CKS(run_sub(false, &redo));
+            CKS(run_sub(false, false, &redo));
         }
     }
     if (prof) {

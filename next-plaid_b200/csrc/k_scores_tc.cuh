@@ -489,7 +489,9 @@ k_cells_emit(const uint32_t *__restrict__ ulist, const int *__restrict__ n_u, co
 //   k_recheck_dots   thread per pair: the pinned-order dot, atomicMax of its score key into exactmax[b][slot][q]
 //   k_recheck_sum    warp per doc: the q-ordered fp32 sum of the maxima -> approx[b][i] and the cut key (what k_approx
 //                    emits); clears the doc's exactmax row for the next call
-// More docs than rc_cap or more pairs than pair_cap raise *fallback (the sub-batch is redone on the exact path).
+// More docs than rc_cap or more pairs than pair_cap raise *fallback (the sub-batch is redone on the exact path).  The
+// abandoned pass must stay memory-safe: k_recheck_sum still gives every candidate a cut key holding its own doc id
+// (score 0 past rc_cap, where no maxima row exists), because k_cut and the exact stage index documents by that id.
 // ------------------------------------------------------------------------------------------
 // Two passes over the doc's codes with the row-group gather of k_approx16 (16-byte loads of 8 query tokens, packed
 // vmaxu2 / vcmpgeu2): pass A the column maxima, pass B (rows now in L1) every (code, query token) whose estimate code is
@@ -656,11 +658,11 @@ k_recheck_sum(uint32_t *__restrict__ exactmax, const int *__restrict__ q_off, in
               u64 *__restrict__ keys, uint32_t doc_id_base) {
     const int b = blockIdx.y, lane = threadIdx.x & 31;
     const int nq = q_off[b + 1] - q_off[b];
-    const int n = min(n_cand[b], rc_cap);
+    const int n = n_cand[b];
     for (int i = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); i < n; i += gridDim.x * (blockDim.x >> 5)) {
         uint32_t *row = exactmax + ((size_t)b * rc_cap + i) * QS;
         float score = 0.0f;  // score += max for q ascending, skipping rows without a finite maximum (search.rs:318-320)
-        for (int qc = 0; qc < QS; qc += 32) {
+        for (int qc = 0; i < rc_cap && qc < QS; qc += 32) {  // past rc_cap the query is flagged: a placeholder key
             const uint32_t mk = qc + lane < QS ? row[qc + lane] : 0u;
             if (qc + lane < QS) row[qc + lane] = 0u;
             const int lim = min(32, nq - qc);

@@ -185,7 +185,8 @@ class ShardGroup:
     """pb_shard_group: several shard handles of ONE process searched together (one host thread per shard).
 
     `search_batch` runs the collective from len(shards) threads and returns rank 0's result (every rank's
-    result is identical; `all_results` keeps them for the tests)."""
+    result is identical; `all_results` keeps them for the tests).  Work counters are per host thread, so each
+    rank's thread also records its `last_work_counters()` in `all_counters`."""
 
     def __init__(self, shards: Sequence["MmapIndex"]):
         self.shards = list(shards)
@@ -195,14 +196,17 @@ class ShardGroup:
         for r, s in enumerate(self.shards):
             _check(load_library().pb_index_group_join(s._h, self._g, r))
         self.all_results = None
+        self.all_counters = None
 
     def search_batch(self, queries, params=None, subset=None):
         import threading
         out, err = [None] * len(self.shards), [None] * len(self.shards)
+        counters = [None] * len(self.shards)
 
         def run(r):
             try:
                 out[r] = self.shards[r].search_batch(queries, params, subset=subset)
+                counters[r] = self.shards[r].last_work_counters()
             except Exception as e:      # noqa: BLE001 - re-raised below
                 err[r] = e
         ths = [threading.Thread(target=run, args=(r,)) for r in range(len(self.shards))]
@@ -212,6 +216,7 @@ class ShardGroup:
             if e is not None:
                 raise e
         self.all_results = out
+        self.all_counters = counters
         return out[0]
 
     def close(self):

@@ -1,7 +1,12 @@
 """Reference implementation of the doc-sharded search protocol (SURVEY.md 8e, DESIGN.md 5) over
 torch.distributed, with the CPU oracle as each shard's engine.  The CUDA path implements the same two
 exchanges with NCCL all-gathers inside libplaid_b200 (k_cut -> all-gather -> k_merge_cut -> k_exact ->
-all-gather -> k_merge_topk); this file is the executable specification the gloo tests run."""
+all-gather -> k_merge_topk); this file is the executable specification the gloo tests run.
+
+The oracle engine never gives a pass up; the CUDA engine's tensor-core pass can, and the redo is collective: each rank's
+local fallback flag (0 on a rank that is not on the tensor-core path) is all-gathered before exchange 1, and if any
+rank raised it, all ranks redo the sub-batch on the exact path together; the ranks also agree on one sub-batch size per
+call.  So every rank issues the same exchanges in the same order."""
 import numpy as np
 
 
@@ -14,9 +19,13 @@ def total_key(scores):
 
 
 def make_shard(oracle, ix, g, G):
-    """Contiguous doc range [d0, d1) of `ix` as its own index: centroids replicated, IVF restricted."""
+    """Shard g of G: the g-th of G contiguous, equal doc ranges of `ix` (shard_range)."""
     D = ix.num_documents
-    d0, d1 = g * D // G, (g + 1) * D // G
+    return shard_range(oracle, ix, g * D // G, (g + 1) * D // G)
+
+
+def shard_range(oracle, ix, d0, d1):
+    """Contiguous doc range [d0, d1) of `ix` as its own index: centroids replicated, IVF restricted."""
     t0, t1 = int(ix.doc_offsets[d0]), int(ix.doc_offsets[d1])
     codes, res, dl = ix.codes[t0:t1], ix.residuals[t0:t1], ix.doc_lengths[d0:d1]
     ivf, ivf_lengths = oracle.build_ivf(codes, dl, ix.num_centroids)
