@@ -278,7 +278,6 @@ struct Stats {
     pb_work_counters work = {};
 };
 static thread_local Stats g_stats;
-static thread_local int g_budget_div = 1;  // lanes of the current call share the workspace budget
 
 // One helper thread of a laned search call (search_impl): runs the pipeline of a slice of the batch on its own workspace
 // and stream while the caller runs another slice, so that one slice's latency-bound kernels overlap the other's
@@ -364,22 +363,37 @@ struct pb_index {
     int rank = 0, world = 1;
     std::mutex mu;
     std::vector<std::unique_ptr<Workspace>> pool;
+};
 
-    pb_status acquire(std::unique_ptr<Workspace> &ws) {
+// A workspace of the handle's pool, held for one call.  It goes back to the pool only if the call set `done`: the
+// kernels restore its scratch invariants (cleared bitmaps, zeroed maxima) as they go, so after a call that failed half
+// way its state is unknown, and it is freed instead once its stream is idle.
+struct WorkspaceLease {
+    pb_index *ix;
+    std::unique_ptr<Workspace> ws;
+    bool done = false;
+    pb_status acquire() {
         {
-            std::lock_guard<std::mutex> g(mu);
-            if (!pool.empty()) {
-                ws = std::move(pool.back());
-                pool.pop_back();
+            std::lock_guard<std::mutex> g(ix->mu);
+            if (!ix->pool.empty()) {
+                ws = std::move(ix->pool.back());
+                ix->pool.pop_back();
                 return PB_OK;
             }
         }
-        ws.reset(new Workspace());
-        return ws->init();
+        std::unique_ptr<Workspace> fresh(new Workspace());
+        CKS(fresh->init());
+        ws = std::move(fresh);
+        return PB_OK;
     }
-    void release(std::unique_ptr<Workspace> &ws) {
-        std::lock_guard<std::mutex> g(mu);
-        pool.push_back(std::move(ws));
+    ~WorkspaceLease() {
+        if (!ws) return;
+        if (done) {
+            std::lock_guard<std::mutex> g(ix->mu);
+            ix->pool.push_back(std::move(ws));
+        } else {
+            cudaStreamSynchronize(ws->stream);
+        }
     }
 };
 
@@ -394,6 +408,22 @@ struct pb_index {
         case 128: { constexpr int DIM = 128; __VA_ARGS__; } break;                                 \
         case 256: { constexpr int DIM = 256; __VA_ARGS__; } break;                                 \
         default: return pb_fail(PB_ERR_UNSUPPORTED, "embedding_dim %d not built (32/64/96/128/256)", dim); \
+    }
+// the dims of the tensor-core kernels
+#define PB_TC_DIM_SWITCH(dim, ...)                                                                 \
+    switch (dim) {                                                                                 \
+        case 64: { constexpr int DIM = 64; __VA_ARGS__; } break;                                   \
+        case 96: { constexpr int DIM = 96; __VA_ARGS__; } break;                                   \
+        case 128: { constexpr int DIM = 128; __VA_ARGS__; } break;                                 \
+        default: return pb_fail(PB_ERR_UNSUPPORTED, "tensor-core kernels: embedding_dim %d not built (64/96/128)", dim); \
+    }
+// bits per residual dimension (a divisor of 8, checked at open)
+#define PB_NBITS_SWITCH(nbits, ...)                                                                \
+    switch (nbits) {                                                                               \
+        case 1: { constexpr int NBITS = 1; __VA_ARGS__; } break;                                   \
+        case 2: { constexpr int NBITS = 2; __VA_ARGS__; } break;                                   \
+        case 4: { constexpr int NBITS = 4; __VA_ARGS__; } break;                                   \
+        default: { constexpr int NBITS = 8; __VA_ARGS__; } break;                                  \
     }
 
 // QS: query tokens per score-table row.  Up to 32 tokens: rounded up to 8 (rows of at most 64 bytes); beyond: to a
@@ -657,11 +687,11 @@ pb_status pb_index_finalize(pb_index *ix) {
         CKS(ix->tok_inv_norm.ensure((size_t)ix->N * 4));  // 1 / |c + w| per token: operand of the linear estimate (k_maxsim_tc)
         const float init[2] = {3.0e38f, 0.0f};
         CK(cudaMemcpy(mn.p, init, 8, cudaMemcpyHostToDevice));
-        switch (ix->dim) {
-            case 64: k_min_vnorm<64><<<ix->sm_count * 8, 256>>>(ix->centroids.as<float>(), ix->w_rev.as<float>(), ix->nbits, ix->codes.as<uint32_t>(), ix->residuals.as<uint8_t>(), ix->N, mn.as<float>(), ix->tok_inv_norm.as<float>()); break;
-            case 96: k_min_vnorm<96><<<ix->sm_count * 8, 256>>>(ix->centroids.as<float>(), ix->w_rev.as<float>(), ix->nbits, ix->codes.as<uint32_t>(), ix->residuals.as<uint8_t>(), ix->N, mn.as<float>(), ix->tok_inv_norm.as<float>()); break;
-            default: k_min_vnorm<128><<<ix->sm_count * 8, 256>>>(ix->centroids.as<float>(), ix->w_rev.as<float>(), ix->nbits, ix->codes.as<uint32_t>(), ix->residuals.as<uint8_t>(), ix->N, mn.as<float>(), ix->tok_inv_norm.as<float>()); break;
-        }
+        PB_TC_DIM_SWITCH(ix->dim, {
+            k_min_vnorm<DIM><<<ix->sm_count * 8, 256>>>(ix->centroids.as<float>(), ix->w_rev.as<float>(), ix->nbits,
+                                                        ix->codes.as<uint32_t>(), ix->residuals.as<uint8_t>(), ix->N,
+                                                        mn.as<float>(), ix->tok_inv_norm.as<float>());
+        });
         CK(cudaGetLastError());
         if ((ix->k1_diag || ix->k1_tc) && ix->cmax > 0.0f && ix->cmax < 3.0e38f) {
             // operands of the tensor-core score table: centroids * 2^cent_exp (max norm in [1, 2)), fp16 hi / lo parts
@@ -796,7 +826,11 @@ extern "C" pb_status pb_last_work_counters(pb_index *, pb_work_counters *out) {
 // ------------------------------------------------------------------------------------------
 // kernel launch helpers shared by the search pipeline and the stage entry points
 // ------------------------------------------------------------------------------------------
-static pb_status launch_centroid_scores_exact(pb_index *ix, Workspace &ws, int B, int QS, int *launches, bool with16);
+static int pow2_ceil(int n) {
+    int P = 1;
+    while (P < n) P <<= 1;
+    return P;
+}
 
 // a2 on the tensor cores (k_scores_tc.cuh).  err = certified bound of |exact - estimate| in 16-bit code units
 // (derivation at the top of that file); E = ceil(err) is the largest difference between an estimate-built code and
@@ -825,23 +859,15 @@ static pb_status launch_k1_table(pb_index *ix, Workspace &ws, int B, int QS, uns
                                                             ws.qrange_tc.as<float2>());
     const int tiles = (int)((ix->K + 127) / 128);
     const size_t sm = (size_t)6 * 128 * ix->dim * 2 + 128;
-#define PB_K1_LAUNCH(DV)                                                                                               \
-    {                                                                                                                  \
-        auto kern = k_scores16_tc<DV>;                                                                                 \
-        CKS(set_smem(kern, sm));                                                                                       \
-        KEV_BEGIN(PB_KERNEL_SCORES);                                                                                   \
-        kern<<<tiles, 320, sm, ws.stream>>>(ix->cent_h16t.as<__half>(), ix->cent_l16t.as<__half>(), ix->K,             \
-                                            ws.Qh16t.as<__half>(), ws.Ql16t.as<__half>(), n_groups, B, QS,             \
-                                            ws.qoff.as<int>(), ws.qrange_tc.as<float2>(), table, flags);               \
-        KEV_END(PB_KERNEL_SCORES);                                                                                     \
-    }
-    switch (ix->dim) {
-        case 64: PB_K1_LAUNCH(64) break;
-        case 96: PB_K1_LAUNCH(96) break;
-        case 128: PB_K1_LAUNCH(128) break;
-        default: return pb_fail(PB_ERR_UNSUPPORTED, "tensor-core score table: dim must be 64, 96 or 128");
-    }
-#undef PB_K1_LAUNCH
+    PB_TC_DIM_SWITCH(ix->dim, {
+        auto kern = k_scores16_tc<DIM>;
+        CKS(set_smem(kern, sm));
+        KEV_BEGIN(PB_KERNEL_SCORES);
+        kern<<<tiles, 320, sm, ws.stream>>>(ix->cent_h16t.as<__half>(), ix->cent_l16t.as<__half>(), ix->K,
+                                            ws.Qh16t.as<__half>(), ws.Ql16t.as<__half>(), n_groups, B, QS,
+                                            ws.qoff.as<int>(), ws.qrange_tc.as<float2>(), table, flags);
+        KEV_END(PB_KERNEL_SCORES);
+    });
     CK(cudaGetLastError());
     return PB_OK;
 }
@@ -868,79 +894,47 @@ static int probe_chunk_rows(long long K, int n, int *n_chunks) {
     return rows;
 }
 
-// a2 + a3 on the tensor-core table.  Nothing is read back here: a flagged query or a probe-list overflow raises
-// *d_fallback on the device, the kernels after it stay memory-safe, and the caller redoes the sub-batch on the
-// exact path once it sees the flag at the end.
-static pb_status run_k1_tc(pb_index *ix, Workspace &ws, const pb_search_params *p, int B, int QS, int nq_max, int n,
-                           bool batched, int *L, int *cells_cap_out, const int **d_fallback_out) {
-    int n_chunks = 0;
-    const int chunk_rows = probe_chunk_rows(ix->K, n, &n_chunks);
-    const int cm = 2 * ix->k1_margin + 1;
-    CKS(ws.Qi.ensure((size_t)B * QS * ix->dim * 4));
-    k_interleave_query_rows<<<dim3(8, B), 256, 0, ws.stream>>>(ws.Q.as<float>(), ws.qoff.as<int>(), QS, ix->dim, ws.Qi.as<float>());
-    CKS(launch_k1_table(ix, ws, B, QS, ws.ST16.as<unsigned short>(), ws.qflag.as<int>()));
-    L[PB_STAGE_CENTROID_SCORES] += 4;
+// The threshold-first probe on the 16-bit table ws.ST16: the largest code of each chunk of centroids per query token,
+// tau = the n-th largest of those, every centroid at or above tau into a per-row list, the top n of each list into
+// ws.sel.  A row that cannot trust its list raises the returned device flag.  On the tensor-core table (tc) the
+// collect settles the codes within the margin around tau by exact dots, and the merge runs whatever the flag says,
+// since k_cells_unique reads every row of sel.  On the exact path the collect reads the fp32 table ws.ST, and the merge
+// leaves sel to the per-lane list scan when the flag is up.
+static pb_status launch_threshold_probe(pb_index *ix, Workspace &ws, int B, int QS, int n, int n_chunks, int chunk_rows,
+                                        bool tc, int **d_fallback_out) {
     const int cap = n * std::max(2, 128 / n);
-    const int cells_cap = (int)std::min<long long>((long long)QS * n, ix->K);
     CKS(ws.cmax16.ensure((size_t)B * n_chunks * QS * 2));
     CKS(ws.tau16.ensure((size_t)B * QS * 4));
     CKS(ws.plist.ensure((size_t)B * QS * cap * 8));
     CKS(ws.pcount.ensure((size_t)B * QS * 4 + 16));
-    CKS(ws.sel.ensure((size_t)B * QS * n * 8));
-    CKS(ws.cells.ensure((size_t)B * cells_cap * 4));
-    CKS(ws.ncells.ensure((size_t)B * 4 + 16));
-    CKS(ws.ulist.ensure((size_t)B * cells_cap * 4));
-    CKS(ws.nulist.ensure((size_t)B * 4 + 16));
-    CKS(ws.k1rows.ensure((size_t)B * cells_cap * QS * 4));
     CK(cudaMemsetAsync(ws.plist.p, 0, (size_t)B * QS * cap * 8, ws.stream));
     CK(cudaMemsetAsync(ws.pcount.p, 0, (size_t)B * QS * 4 + 16, ws.stream));
     int *d_fallback = ws.pcount.as<int>() + (size_t)B * QS;
-    k_chunkmax16<<<dim3((n_chunks + 3) / 4, B), 128, 0, ws.stream>>>(ws.ST16.as<unsigned short>(), ix->K, QS, n_chunks,
-                                                                     chunk_rows, ws.cmax16.as<unsigned short>());
+    const dim3 grid((n_chunks + 3) / 4, B);
+    k_chunkmax16<<<grid, 128, 0, ws.stream>>>(ws.ST16.as<unsigned short>(), ix->K, QS, n_chunks, chunk_rows,
+                                              ws.cmax16.as<unsigned short>());
     k_tau16<<<dim3(QS, B), 32, 0, ws.stream>>>(ws.cmax16.as<unsigned short>(), ws.qoff.as<int>(), QS, n, n_chunks,
                                               ws.qflag.as<int>(), ws.tau16.as<uint32_t>(), d_fallback);
-    k_collect16_tc<<<dim3((n_chunks + 3) / 4, B), 128, 0, ws.stream>>>(
-        ws.ST16.as<unsigned short>(), ws.Q.as<float>(), ws.qoff.as<int>(), ix->centroids.as<float>(), ix->dim, cm, ix->K, QS,
-        n_chunks, chunk_rows, ws.tau16.as<uint32_t>(), cap, ws.pcount.as<int>(), ws.plist.as<u64>(), d_fallback);
+    if (tc)
+        k_collect16_tc<<<grid, 128, 0, ws.stream>>>(ws.ST16.as<unsigned short>(), ws.Q.as<float>(), ws.qoff.as<int>(),
+                                                    ix->centroids.as<float>(), ix->dim, 2 * ix->k1_margin + 1, ix->K, QS,
+                                                    n_chunks, chunk_rows, ws.tau16.as<uint32_t>(), cap, ws.pcount.as<int>(),
+                                                    ws.plist.as<u64>(), d_fallback);
+    else
+        k_collect16<<<grid, 128, 0, ws.stream>>>(ws.ST16.as<unsigned short>(), ws.ST.as<float>(), ix->K, QS, n_chunks,
+                                                 chunk_rows, ws.tau16.as<uint32_t>(), cap, ws.pcount.as<int>(),
+                                                 ws.plist.as<u64>(), d_fallback);
     k_topn_merge<<<dim3(QS, B), 32, 0, ws.stream>>>(ws.plist.as<u64>(), ws.qoff.as<int>(), QS, n, cap / n, ws.sel.as<u64>(),
-                                                  nullptr, 0);
-    // the selected centroids, their exact rows, the variant's threshold rule
-    int P = 1;
-    while (P < std::max(nq_max * n, 1)) P <<= 1;
-    CKS(set_smem(k_cells_unique, (size_t)P * 8));
-    k_cells_unique<<<B, 256, (size_t)P * 8, ws.stream>>>(ws.sel.as<u64>(), ws.qoff.as<int>(), QS, n, cells_cap,
-                                                         ws.ulist.as<uint32_t>(), ws.nulist.as<int>());
-    const size_t smr = (size_t)(PB_TOK_TILE * (ix->dim + 4) + PB_Q_TILE * ix->dim) * sizeof(float);
-    PB_DIM_SWITCH(ix->dim, {
-        auto kern = k_exact_rows<DIM>;
-        CKS(set_smem(kern, smr));
-        kern<<<dim3((cells_cap + PB_TOK_TILE - 1) / PB_TOK_TILE, B), 128, smr, ws.stream>>>(
-            ws.Qi.as<float>(), ws.qoff.as<int>(), QS, ix->centroids.as<float>(), ws.ulist.as<uint32_t>(), ws.nulist.as<int>(),
-            cells_cap, ws.k1rows.as<float>());
-    });
-    CKS(ws.cellflags.ensure((size_t)B * cells_cap * 4));
-    k_cells_thr<<<dim3(8, B), 256, 0, ws.stream>>>(
-        ws.sel.as<u64>(), ws.k1rows.as<float>(), ws.ulist.as<uint32_t>(), ws.nulist.as<int>(), ws.qoff.as<int>(), ix->K, QS, n,
-        cells_cap, p->has_centroid_score_threshold, p->centroid_score_threshold, batched ? 1 : 0,
-        batched ? (long long)p->centroid_batch_size : ix->K, ws.cellflags.as<int>(), ws.ST16.as<unsigned short>(),
-        ws.qrange.as<float2>(), cm, ws.Q.as<float>(), ix->centroids.as<float>(), ix->dim, ws.cmax16.as<unsigned short>(),
-        n_chunks, chunk_rows);
-    k_cells_emit<<<B, 256, 0, ws.stream>>>(ws.ulist.as<uint32_t>(), ws.nulist.as<int>(), ws.cellflags.as<int>(), cells_cap,
-                                           ws.cells.as<uint32_t>(), ws.ncells.as<int>());
+                                                  tc ? nullptr : d_fallback, 0);
     CK(cudaGetLastError());
-    L[PB_STAGE_PROBE] += 8;
-    *cells_cap_out = cells_cap;
+    g_stats.launches[PB_STAGE_PROBE] += 4;
     *d_fallback_out = d_fallback;
     return PB_OK;
 }
 
-static pb_status launch_centroid_scores(pb_index *ix, Workspace &ws, int B, int QS, int *launches, bool with16 = false) {
-    CKS(launch_centroid_scores_exact(ix, ws, B, QS, launches, with16));
-    if (with16 && ix->k1_diag && ix->cent_h16t.p) CKS(launch_k1_diag(ix, ws, B, QS));
-    return PB_OK;
-}
-
-static pb_status launch_centroid_scores_exact(pb_index *ix, Workspace &ws, int B, int QS, int *launches, bool with16) {
+// a2 on the exact fp32 kernel: the table ws.ST and, with16, its 16-bit twin ws.ST16 (under PB_K1_TC_DIAG also the
+// tensor-core table, compared with it)
+static pb_status launch_centroid_scores(pb_index *ix, Workspace &ws, int B, int QS, int *launches, bool with16) {
     const int tiles = (int)((ix->K + PB_TOK_TILE - 1) / PB_TOK_TILE);
     // enough CTAs to fill the machine twice over; each CTA keeps its centroid tile in smem and walks queries
     int groups = std::max(1, std::min(B, (4 * ix->sm_count + tiles - 1) / tiles));
@@ -961,6 +955,7 @@ static pb_status launch_centroid_scores_exact(pb_index *ix, Workspace &ws, int B
     });
     CK(cudaGetLastError());
     if (launches) *launches += 2;
+    if (with16 && ix->k1_diag && ix->cent_h16t.p) CKS(launch_k1_diag(ix, ws, B, QS));
     return PB_OK;
 }
 
@@ -1091,41 +1086,19 @@ static pb_status launch_maxsim_tc(pb_index *ix, Workspace &ws, const KeptView &i
     k_doc_gbase<<<dim3((Mcap + 255) / 256, B), 256, 0, ws.stream>>>(in.kept, in.nkept, in.tokp, ix->doc_off.as<long long>(), Mcap,
                                                                     ws.gbase.as<long long>());
     CK(cudaGetLastError());
-#define PB_MS_GO(DV, NB, NQ, EM)                                                                                       \
-    {                                                                                                                  \
-        auto kern = k_maxsim_tc<DV, NB, NQ, EM>;                                                                       \
-        CKS(set_smem(kern, sm));                                                                                       \
-        if (kev >= 0) KEV_BEGIN(kev);                                                                                  \
-        kern<<<dim3(gx, B), 288, sm, ws.stream>>>(ws.Q.as<float>(), ws.qoff.as<int>(), QS, ws.ST16.as<unsigned short>(), \
-                                                  ix->K, ws.qrange.as<float2>(), ws.qflag.as<int>(), ix->w_rev.as<float>(), \
-                                                  ix->codes.as<uint32_t>(), ix->residuals.as<uint8_t>(),               \
-                                                  ix->tok_inv_norm.as<float>(), ws.gbase.as<long long>(),              \
-                                                  in.nkept, in.tokp, Mcap, keys, src_rank, ws.qnmax.as<float>(),       \
-                                                  band_unit, pairs, n_pairs, pair_cap);                                \
-        if (kev >= 0) KEV_END(kev);                                                                                    \
-    }
-#define PB_MS_LAUNCH(DV, NB)                                                                                           \
-    if (emit) {                                                                                                        \
-        if (nqt == 32) PB_MS_GO(DV, NB, 32, true) else PB_MS_GO(DV, NB, 64, true)                                      \
-    } else {                                                                                                           \
-        if (nqt == 32) PB_MS_GO(DV, NB, 32, false) else PB_MS_GO(DV, NB, 64, false)                                    \
-    }
-#define PB_MS_NBITS(DV)                                                                                                \
-    switch (ix->nbits) {                                                                                               \
-        case 1: PB_MS_LAUNCH(DV, 1) break;                                                                             \
-        case 2: PB_MS_LAUNCH(DV, 2) break;                                                                             \
-        case 4: PB_MS_LAUNCH(DV, 4) break;                                                                             \
-        default: PB_MS_LAUNCH(DV, 8) break;                                                                            \
-    }
-    switch (ix->dim) {
-        case 64: PB_MS_NBITS(64) break;
-        case 96: PB_MS_NBITS(96) break;
-        case 128: PB_MS_NBITS(128) break;
-        default: return pb_fail(PB_ERR_UNSUPPORTED, "filter: unsupported dim");
-    }
-#undef PB_MS_NBITS
-#undef PB_MS_LAUNCH
-#undef PB_MS_GO
+    PB_TC_DIM_SWITCH(ix->dim, PB_NBITS_SWITCH(ix->nbits, {
+        auto kern = emit ? (nqt == 32 ? k_maxsim_tc<DIM, NBITS, 32, true> : k_maxsim_tc<DIM, NBITS, 64, true>)
+                         : (nqt == 32 ? k_maxsim_tc<DIM, NBITS, 32, false> : k_maxsim_tc<DIM, NBITS, 64, false>);
+        CKS(set_smem(kern, sm));
+        if (kev >= 0) KEV_BEGIN(kev);
+        kern<<<dim3(gx, B), 288, sm, ws.stream>>>(ws.Q.as<float>(), ws.qoff.as<int>(), QS, ws.ST16.as<unsigned short>(),
+                                                  ix->K, ws.qrange.as<float2>(), ws.qflag.as<int>(), ix->w_rev.as<float>(),
+                                                  ix->codes.as<uint32_t>(), ix->residuals.as<uint8_t>(),
+                                                  ix->tok_inv_norm.as<float>(), ws.gbase.as<long long>(),
+                                                  in.nkept, in.tokp, Mcap, keys, src_rank, ws.qnmax.as<float>(),
+                                                  band_unit, pairs, n_pairs, pair_cap);
+        if (kev >= 0) KEV_END(kev);
+    }));
     CK(cudaGetLastError());
     return PB_OK;
 }
@@ -1146,39 +1119,22 @@ static pb_status launch_filter(pb_index *ix, Workspace &ws, const KeptView &in, 
         CKS(launch_maxsim_tc(ix, ws, in, B, QS, Mcap, max_tokens, nq_max, keys, nullptr, 0.0f, nullptr, nullptr, 0,
                              PB_KERNEL_FILTER));
     } else {
-#define PB_TC_LAUNCH(DV, NB)                                                                                           \
-    {                                                                                                                  \
-        auto kern = nqt == 32 ? k_exact_tc<DV, NB, 32> : k_exact_tc<DV, NB, 64>;                                       \
-        CKS(set_smem(kern, sm));                                                                                       \
-        KEV_BEGIN(PB_KERNEL_FILTER);                                                                                   \
-        kern<<<dim3(gx, B), 128, sm, ws.stream>>>(ws.Q.as<float>(), ws.qoff.as<int>(), QS,                             \
-                                                  ix->centroids_f16.as<__half>(), ix->w_rev.as<float>(),               \
-                                                  ix->codes.as<uint32_t>(), ix->residuals.as<uint8_t>(),               \
-                                                  ix->doc_off.as<long long>(), in.kept, in.nkept, in.tokp, Mcap, keys); \
-        KEV_END(PB_KERNEL_FILTER);                                                                                     \
-    }
-#define PB_TC_NBITS(DV)                                                                                                \
-    switch (ix->nbits) {                                                                                               \
-        case 1: PB_TC_LAUNCH(DV, 1) break;                                                                             \
-        case 2: PB_TC_LAUNCH(DV, 2) break;                                                                             \
-        case 4: PB_TC_LAUNCH(DV, 4) break;                                                                             \
-        default: PB_TC_LAUNCH(DV, 8) break;                                                                            \
-    }
-        switch (ix->dim) {
-            case 64: PB_TC_NBITS(64) break;
-            case 96: PB_TC_NBITS(96) break;
-            case 128: PB_TC_NBITS(128) break;
-            default: return pb_fail(PB_ERR_UNSUPPORTED, "filter: unsupported dim");
-        }
-#undef PB_TC_NBITS
-#undef PB_TC_LAUNCH
+        PB_TC_DIM_SWITCH(ix->dim, PB_NBITS_SWITCH(ix->nbits, {
+            auto kern = nqt == 32 ? k_exact_tc<DIM, NBITS, 32> : k_exact_tc<DIM, NBITS, 64>;
+            CKS(set_smem(kern, sm));
+            KEV_BEGIN(PB_KERNEL_FILTER);
+            kern<<<dim3(gx, B), 128, sm, ws.stream>>>(ws.Q.as<float>(), ws.qoff.as<int>(), QS,
+                                                      ix->centroids_f16.as<__half>(), ix->w_rev.as<float>(),
+                                                      ix->codes.as<uint32_t>(), ix->residuals.as<uint8_t>(),
+                                                      ix->doc_off.as<long long>(), in.kept, in.nkept, in.tokp, Mcap, keys);
+            KEV_END(PB_KERNEL_FILTER);
+        }));
         CK(cudaGetLastError());
     }
     k_tc_finalize<<<dim3((Mcap + 7) / 8, B), 256, 0, ws.stream>>>(keys, ws.qoff.as<int>(), QS, in.nkept, Mcap, in.tokp,
                                                                   ws.est.as<float>(), keep_keys ? 0 : 1);
     CK(cudaGetLastError());
-    int Pm = 1;
-    while (Pm < Mcap) Pm <<= 1;
+    const int Pm = pow2_ceil(Mcap);
     CKS(set_smem(k_tc_select, (size_t)Pm * 8));
     k_tc_select<<<B, 1024, (size_t)Pm * 8, ws.stream>>>(ws.est.as<float>(), in.kept, in.krank, in.nkept, Mcap, top_k,
                                                         ws.qoff.as<int>(), ws.qnmax.as<float>(), eps_unit,
@@ -1191,7 +1147,8 @@ static pb_status launch_filter(pb_index *ix, Workspace &ws, const KeptView &in, 
 }
 
 // ------------------------------------------------------------------------------------------
-// the search pipeline
+// the search pipeline: plan_call decides what holds for the whole call, run_pass runs the stages a2..a9 over one
+// sub-batch (stage_* below, in pipeline order), search_impl_inner loops over the sub-batches
 // ------------------------------------------------------------------------------------------
 struct SearchIO {
     const float *queries;  // host or device
@@ -1208,7 +1165,125 @@ struct SearchIO {
     pb_trace *trace;
 };
 
-static pb_status search_impl_inner(pb_index *ix, const pb_search_params *p, const SearchIO &io) {
+struct CallPlan {
+    const pb_search_params *p = nullptr;
+    const SearchIO *io = nullptr;
+    int64_t Bt = 0;                  // queries of the call
+    bool empty = false;              // every result is empty: no sub-batch runs
+    int top_k = 0, M = 0, Mcap = 1;  // M: docs the cut keeps, min(n_full_scores, max(n_full_scores / 4, top_k))
+    bool batched = false, sharded = false;
+    bool fast = false;               // two-pass approximate stage on a 16-bit table
+    long long Wd = 0, Wk = 0;        // 32-bit words of a doc / centroid bitmap
+    const uint32_t *d_subset_bits = nullptr, *d_elig = nullptr;
+    int n_probe = 0;
+    long long n_elig = 0;
+    bool all_eligible = false, big_probe = false;
+    bool tc_call = false;            // a sub-batch whose rows fit (QS / 8 <= 32) takes the tensor-core path
+    int QB = 1;                      // queries per sub-batch
+};
+
+// how a3 picks the cells of each query token
+enum class ProbeMode {
+    TensorCore,   // threshold-first on the estimate table, done by run_k1_tc in a2
+    Threshold,    // threshold-first on the 16-bit table; the per-lane list scan where the device raises the fallback flag
+    List,         // per-lane list scan of the fp32 table
+    AllEligible,  // every eligible centroid (a subset whose scaled n_ivf_probe reaches them all)
+    BigProbe,     // row-wise radix select (n_ivf_probe beyond the per-lane lists)
+};
+
+// The pinned host buffer of one pass (ws.hcounts): the query offsets going to the device, and the per-query counts,
+// work counters and flags coming back
+struct PassHost {
+    int *qoff;                     // [B + 1]
+    unsigned long long *counters;  // [B + 2] ws.counters: candidate codes gathered, kept-doc tokens per query, re-check gathers
+    long long *surv_tokens;        // [B] tokens of the filter's survivors
+    int *n_cells, *n_cand, *n_kept, *survivors, *rechecked, *pairs, *need_exact;  // [B] each
+    int *fell;                     // the threshold-first probe gave up
+    // lays the fields out from `base`, 16-byte aligned, and returns their size (base == nullptr: only the size)
+    size_t carve(char *base, int B) {
+        size_t off = 0;
+        auto at = [&](size_t bytes) {
+            off = (off + 15) & ~(size_t)15;
+            char *q = base ? base + off : nullptr;
+            off += bytes;
+            return q;
+        };
+        qoff = reinterpret_cast<int *>(at((size_t)(B + 1) * 4));
+        counters = reinterpret_cast<unsigned long long *>(at((size_t)(B + 2) * 8));
+        surv_tokens = reinterpret_cast<long long *>(at((size_t)B * 8));
+        for (int **f : {&n_cells, &n_cand, &n_kept, &survivors, &rechecked, &pairs, &need_exact})
+            *f = reinterpret_cast<int *>(at((size_t)B * 4));
+        fell = reinterpret_cast<int *>(at(4));
+        return off;
+    }
+};
+
+// One pass over the sub-batch [b0, b0 + B): its shape (H2D), then what each stage decides for the stages after it
+struct Pass {
+    int64_t b0 = 0, r0 = 0, R = 0;  // first query, its first token, the sub-batch's tokens
+    int B = 0, nq_max = 0, QS = 0;
+    bool tc = false;                // a2 + a3 on the tensor-core table
+    ProbeMode probe = ProbeMode::List;
+    int cells_cap = 0;              // a3: cells per query
+    int *d_fallback = nullptr;      // a3: device flag of the threshold-first probe (0 = it did the work)
+    const uint32_t *cand_list = nullptr;  // a5: the candidates scored, which the cut reads
+    const int *cand_n = nullptr;
+    KeptView kv = {};               // a6 / a7: the docs the exact stage scores
+    bool filt = false;              // a7: the certified filter ran
+    bool pairs = false;             // a8: the exact stage ran on (token, query token) pairs
+    long long *d_ids = nullptr;     // a9: the results on the device
+    float *d_sc = nullptr;
+    int *d_cn = nullptr;
+    PassHost host = {};
+};
+
+// The subset of a call: its doc bitmap and, with the dense variant, the eligible centroids and the scaled n_ivf_probe
+// (search.rs:350-382).  No eligible centroid: every per-token pool is empty, so every result is (plan.empty).
+static pb_status plan_subset(pb_index *ix, Workspace &ws, const SearchIO &io, CallPlan &plan) {
+    const pb_search_params *p = plan.p;
+    CKS(ws.subset_bits.ensure((size_t)plan.Wd * 4));
+    CK(cudaMemsetAsync(ws.subset_bits.p, 0, (size_t)plan.Wd * 4, ws.stream));
+    if (io.n_subset > 0) {
+        CKS(ws.subset.ensure((size_t)io.n_subset * 8));
+        CK(cudaMemcpyAsync(ws.subset.p, io.subset, (size_t)io.n_subset * 8, cudaMemcpyHostToDevice, ws.stream));
+        k_subset_bits<<<296, 256, 0, ws.stream>>>(ws.subset.as<long long>(), io.n_subset, ix->doc_id_base, ix->D,
+                                                 ws.subset_bits.as<uint32_t>());
+        CK(cudaGetLastError());
+    }
+    plan.d_subset_bits = ws.subset_bits.as<uint32_t>();
+    if (plan.batched) return PB_OK;
+    CKS(ws.elig.ensure((size_t)plan.Wk * 4));
+    CKS(ws.misc.ensure(64));
+    CK(cudaMemsetAsync(ws.elig.p, 0, (size_t)plan.Wk * 4, ws.stream));
+    CK(cudaMemsetAsync(ws.misc.p, 0, 64, ws.stream));
+    k_eligible_bits<<<ix->sm_count * 8, 256, 0, ws.stream>>>(plan.d_subset_bits, ix->D, ix->doc_off.as<long long>(),
+                                                             ix->codes.as<uint32_t>(), ws.elig.as<uint32_t>());
+    k_popcount<<<ix->sm_count, 256, 0, ws.stream>>>(ws.elig.as<uint32_t>(), plan.Wk, ws.misc.as<unsigned long long>());
+    CK(cudaGetLastError());
+    unsigned long long ne = 0;
+    CK(cudaMemcpyAsync(&ne, ws.misc.p, 8, cudaMemcpyDeviceToHost, ws.stream));
+    CK(cudaStreamSynchronize(ws.stream));
+    plan.n_elig = (long long)ne;
+    if (plan.n_elig == 0) {
+        plan.empty = true;
+        return PB_OK;
+    }
+    unsigned long long scaled = io.n_subset > 0 ? (unsigned long long)p->n_ivf_probe * (unsigned long long)ix->D /
+                                                      (unsigned long long)io.n_subset
+                                                : (unsigned long long)p->n_ivf_probe;
+    scaled = std::max<unsigned long long>(scaled, (unsigned long long)p->n_ivf_probe);
+    scaled = std::min<unsigned long long>(scaled, (unsigned long long)plan.n_elig);
+    plan.d_elig = ws.elig.as<uint32_t>();
+    if ((long long)scaled >= plan.n_elig) plan.all_eligible = true;
+    else plan.n_probe = (int)scaled;
+    return PB_OK;
+}
+
+// Everything a search call decides once: the argument checks, the cut size, the variant, the subset, the probe, whether
+// the tensor-core path is open and the sub-batch size.  Takes the call's workspace from the pool (lease) unless the
+// call has no queries.  `lanes`: concurrent slices of the caller's batch, which share the workspace budget.
+static pb_status plan_call(pb_index *ix, const pb_search_params *p, const SearchIO &io, int lanes, WorkspaceLease &lease,
+                           CallPlan &plan) {
     if (!ix || !p) return pb_fail(PB_ERR_INVALID, "null argument");
     if (io.n_queries < 0) return pb_fail(PB_ERR_INVALID, "n_queries < 0");
     if (io.n_queries > 0 && (!io.queries || !io.q_off)) return pb_fail(PB_ERR_INVALID, "null queries");
@@ -1218,115 +1293,50 @@ static pb_status search_impl_inner(pb_index *ix, const pb_search_params *p, cons
     if (!io.out_counts) return pb_fail(PB_ERR_INVALID, "null out_counts");
     CK(cudaSetDevice(ix->device));
     g_stats = Stats();
-    const int64_t Bt = io.n_queries;
+    plan.p = p;
+    plan.io = &io;
+    const int64_t Bt = plan.Bt = io.n_queries;
     if (Bt == 0) return PB_OK;
     for (int64_t b = 0; b < Bt; ++b)
         if (io.q_off[b + 1] < io.q_off[b]) return pb_fail(PB_ERR_INVALID, "q_tok_offsets not monotone");
-    const int top_k = (int)p->top_k;
+    plan.top_k = (int)p->top_k;
     const long long n_dec = std::max<long long>(p->n_full_scores / 4, p->top_k);  // search.rs:468
     const long long Mll = std::min<long long>(p->n_full_scores, n_dec);             // take(nfs).take(n_dec)
     if (Mll > 16384)
         return pb_fail(PB_ERR_UNSUPPORTED, "min(n_full_scores, max(n_full_scores/4, top_k)) = %lld exceeds 16384", Mll);
-    const int M = (int)Mll;
-    const int Mcap = std::max(M, 1);
-    const bool batched = p->centroid_batch_size > 0 && ix->K > p->centroid_batch_size;  // search.rs:337
-    const bool sharded = ix->world > 1;
-    if (sharded && io.has_subset && !batched)
+    plan.M = (int)Mll;
+    plan.Mcap = std::max(plan.M, 1);
+    plan.batched = p->centroid_batch_size > 0 && ix->K > p->centroid_batch_size;  // search.rs:337
+    plan.sharded = ix->world > 1;
+    if (plan.sharded && io.has_subset && !plan.batched)
         return pb_fail(PB_ERR_UNSUPPORTED, "subset with the dense variant needs the global eligible-centroid set; "
                                             "not built for doc-sharded indices");
+    CKS(lease.acquire());
+    Workspace &ws = *lease.ws;
     // a shard with no documents still takes part in the exchanges
-    const bool empty_all = (M == 0 || top_k == 0 || (ix->D == 0 && !sharded));
+    plan.empty = plan.M == 0 || plan.top_k == 0 || (ix->D == 0 && !plan.sharded);
+    if (plan.empty) return PB_OK;
 
-    std::unique_ptr<Workspace> wsp;
-    CKS(ix->acquire(wsp));
-    Workspace &ws = *wsp;
-    // A workspace goes back to the pool only after a search that ran to completion: its scratch
-    // invariants (cleared bitmaps, zeroed maxima) are restored by the kernels themselves, so a call that
-    // fails half way must not hand its buffers to the next caller.
-    struct Releaser {
-        pb_index *ix;
-        std::unique_ptr<Workspace> &w;
-        bool ok = false;
-        ~Releaser() {
-            if (ok) ix->release(w);
-            else {
-                cudaStreamSynchronize(w->stream);
-                w.reset();
-            }
-        }
-    } rel{ix, wsp};
-
-    auto zero_counts = [&](int64_t b0, int64_t nb) -> pb_status {
-        if (io.out_on_device) CK(cudaMemsetAsync(io.out_counts + b0, 0, (size_t)nb * 4, ws.stream));
-        else memset(io.out_counts + b0, 0, (size_t)nb * 4);
-        return PB_OK;
-    };
-    if (empty_all) {
-        CKS(zero_counts(0, Bt));
-        CK(cudaStreamSynchronize(ws.stream));
-        rel.ok = true;
-        return PB_OK;
-    }
-
-    // ---- subset preparation (shared by every query of the call) ----
-    const long long Wd = (ix->D + 31) / 32, Wk = (ix->K + 31) / 32;
-    const uint32_t *d_subset_bits = nullptr, *d_elig = nullptr;
-    int n_probe = (int)std::min<long long>(p->n_ivf_probe, ix->K);
-    bool all_eligible = false;
-    long long n_elig = 0;
+    plan.Wd = (ix->D + 31) / 32;
+    plan.Wk = (ix->K + 31) / 32;
+    plan.n_probe = (int)std::min<long long>(p->n_ivf_probe, ix->K);
     if (io.has_subset) {
-        CKS(ws.subset_bits.ensure((size_t)Wd * 4));
-        CK(cudaMemsetAsync(ws.subset_bits.p, 0, (size_t)Wd * 4, ws.stream));
-        if (io.n_subset > 0) {
-            CKS(ws.subset.ensure((size_t)io.n_subset * 8));
-            CK(cudaMemcpyAsync(ws.subset.p, io.subset, (size_t)io.n_subset * 8, cudaMemcpyHostToDevice, ws.stream));
-            k_subset_bits<<<296, 256, 0, ws.stream>>>(ws.subset.as<long long>(), io.n_subset, ix->doc_id_base, ix->D,
-                                                     ws.subset_bits.as<uint32_t>());
-            CK(cudaGetLastError());
-        }
-        d_subset_bits = ws.subset_bits.as<uint32_t>();
-        if (!batched) {
-            // eligible centroids + n_ivf_probe scaling, dense variant only (search.rs:350-382)
-            CKS(ws.elig.ensure((size_t)Wk * 4));
-            CKS(ws.misc.ensure(64));
-            CK(cudaMemsetAsync(ws.elig.p, 0, (size_t)Wk * 4, ws.stream));
-            CK(cudaMemsetAsync(ws.misc.p, 0, 64, ws.stream));
-            k_eligible_bits<<<ix->sm_count * 8, 256, 0, ws.stream>>>(d_subset_bits, ix->D, ix->doc_off.as<long long>(),
-                                                                     ix->codes.as<uint32_t>(), ws.elig.as<uint32_t>());
-            k_popcount<<<ix->sm_count, 256, 0, ws.stream>>>(ws.elig.as<uint32_t>(), Wk, ws.misc.as<unsigned long long>());
-            CK(cudaGetLastError());
-            unsigned long long ne = 0;
-            CK(cudaMemcpyAsync(&ne, ws.misc.p, 8, cudaMemcpyDeviceToHost, ws.stream));
-            CK(cudaStreamSynchronize(ws.stream));
-            n_elig = (long long)ne;
-            if (n_elig == 0) {  // every per-token pool is empty -> no cells -> empty results
-                CKS(zero_counts(0, Bt));
-                CK(cudaStreamSynchronize(ws.stream));
-                rel.ok = true;
-                return PB_OK;
-            }
-            unsigned long long scaled = io.n_subset > 0 ? (unsigned long long)p->n_ivf_probe * (unsigned long long)ix->D /
-                                                              (unsigned long long)io.n_subset
-                                                        : (unsigned long long)p->n_ivf_probe;
-            scaled = std::max<unsigned long long>(scaled, (unsigned long long)p->n_ivf_probe);
-            scaled = std::min<unsigned long long>(scaled, (unsigned long long)n_elig);
-            d_elig = ws.elig.as<uint32_t>();
-            if ((long long)scaled >= n_elig) all_eligible = true;
-            else n_probe = (int)scaled;
-        }
+        CKS(plan_subset(ix, ws, io, plan));
+        if (plan.empty) return PB_OK;
     }
     // effective n_ivf_probe beyond 64: the dense variant switches to a row-wise radix select; the batched variant's
     // heap-order threshold rule is tied to the streaming formulation, whose per-lane lists hold up to 192 entries
-    const int stream_max = batched ? 192 : 64;
-    const bool big_probe = !all_eligible && n_probe > stream_max;
-    if (big_probe && batched)
+    const int n_probe = plan.n_probe;
+    const int stream_max = plan.batched ? 192 : 64;
+    plan.big_probe = !plan.all_eligible && n_probe > stream_max;
+    if (plan.big_probe && plan.batched)
         return pb_fail(PB_ERR_UNSUPPORTED, "n_ivf_probe %d > 192 with the batched variant is not built", n_probe);
 
     // ---- sub-batching: bound the transposed score matrix ----
     int nq_max_all = 0;
     for (int64_t b = 0; b < Bt; ++b) nq_max_all = std::max<int>(nq_max_all, (int)(io.q_off[b + 1] - io.q_off[b]));
     const int QS_all = query_row_tokens(nq_max_all);
-    if (!all_eligible && !big_probe && (long long)QS_all * n_probe > 8192)
+    if (!plan.all_eligible && !plan.big_probe && (long long)QS_all * n_probe > 8192)
         return pb_fail(PB_ERR_UNSUPPORTED, "query tokens x n_ivf_probe = %lld exceeds 8192", (long long)QS_all * n_probe);
     size_t per_q = (size_t)ix->K * QS_all * sizeof(float);
     if (per_q >= ((size_t)1 << 32))
@@ -1334,560 +1344,677 @@ static pb_status search_impl_inner(pb_index *ix, const pb_search_params *p, cons
     // the score table comes from the tensor cores unless something needs the dense fp32 S (an eligibility filter,
     // the radix-select probe, a trace) or the shape is outside the kernel's (DESIGN.md "a2"); all of that is fixed for
     // the call except the sub-batch's row width QS / 8 <= 32
-    const bool fast = ix->fast_approx && !io.trace;  // trace wants every candidate's exact approximate score
+    plan.fast = ix->fast_approx && !io.trace;  // trace wants every candidate's exact approximate score
     int n_chunks_k = 0;
     probe_chunk_rows(ix->K, n_probe, &n_chunks_k);
-    const bool tc_call = k1_tc_usable(ix) && fast && ix->probe16 && !ix->k1_diag && !all_eligible && !big_probe && !d_elig &&
-                         n_chunks_k >= n_probe && n_probe <= 192;
+    plan.tc_call = k1_tc_usable(ix) && plan.fast && ix->probe16 && !ix->k1_diag && !plan.all_eligible && !plan.big_probe &&
+                   !plan.d_elig && n_chunks_k >= n_probe && n_probe <= 192;
     // sub-batch size: the score tables (16-bit on the tensor-core path; fp32 and 16-bit otherwise) and the per-(query,
     // doc) scratch (candidate lists, code sums, approximate scores, cut keys, bitmap: 24.2 bytes per document) share
     // one budget
-    const bool tc_all = tc_call && QS_all / 8 <= 32;  // every sub-batch of the call can take the tensor-core path
+    const bool tc_all = plan.tc_call && QS_all / 8 <= 32;  // every sub-batch of the call can take the tensor-core path
     const size_t per_q_all = (size_t)ix->K * QS_all * (tc_all ? 2 : 6) + (size_t)ix->D * 24 + (size_t)ix->D / 8 + 4096;
-    int QB = (int)std::max<size_t>(1, std::min<size_t>((size_t)Bt, ix->st_budget / std::max(g_budget_div, 1) / per_q_all));
+    int QB = (int)std::max<size_t>(1, std::min<size_t>((size_t)Bt, ix->st_budget / lanes / per_q_all));
     QB = std::min(QB, 256);
-    if (sharded) {
+    if (plan.sharded) {
         // every rank must cut the call into the same sub-batches (each sub-batch is a set of exchanges), but per_q_all
         // depends on the shard's own documents and tensor-core operands: the group takes the smallest size
         const u64 *all = nullptr;
         CKS(shard_vote(ix, ws, (u64)QB, nullptr, &all));
         for (int g = 0; g < ix->world; ++g) QB = std::min<int>(QB, (int)all[g]);
     }
-    QB = (int)((Bt + (Bt + QB - 1) / QB - 1) / ((Bt + QB - 1) / QB));  // equal sub-batches
+    plan.QB = (int)((Bt + (Bt + QB - 1) / QB - 1) / ((Bt + QB - 1) / QB));  // equal sub-batches
+    return PB_OK;
+}
 
-    const bool prof = ix->profiling;
-    if (prof) CK(cudaEventRecord(ws.call_ev[0], ws.stream));
-    for (int64_t b0 = 0; b0 < Bt; b0 += QB) {
-        const int B = (int)std::min<int64_t>(QB, Bt - b0);
-        const int64_t r0 = io.q_off[b0];
-        const int64_t R = io.q_off[b0 + B] - r0;
-        int nq_max = 0;
-        std::vector<int> qoff(B + 1);
-        for (int b = 0; b <= B; ++b) qoff[b] = (int)(io.q_off[b0 + b] - r0);
-        for (int b = 0; b < B; ++b) nq_max = std::max(nq_max, qoff[b + 1] - qoff[b]);
-        const int QS = query_row_tokens(nq_max);
-        int *L = g_stats.launches;
-        const bool want_tc = tc_call && QS / 8 <= 32;
-        // One pass over the sub-batch.  use_tc: a flagged query, a probe-list overflow or a re-check overflow raises a
-        // device flag instead of being read back mid-way; the pass then finishes on (memory-safe) garbage and *redo asks
-        // for the exact pass.  vote (a sharded handle's first pass over the sub-batch, on every rank whatever path it
-        // takes): the ranks' flags are gathered before the first exchange, so that every rank abandons the pass
-        // together and the ranks' exchanges stay paired.
-        auto run_sub = [&](const bool use_tc, const bool vote, bool *redo) -> pb_status {
-        *redo = false;
-        if (prof) CK(cudaEventRecord(ws.ev[0], ws.stream));
-        // ---- H2D ----
-        CKS(ws.Q.ensure(std::max<size_t>((size_t)R * ix->dim * 4, 16)));
-        CKS(ws.qoff.ensure((size_t)(B + 1) * 4));
-        if (R > 0) {
-            if (io.queries_on_device)
-                CK(cudaMemcpyAsync(ws.Q.p, io.queries + (size_t)r0 * ix->dim, (size_t)R * ix->dim * 4,
-                                   cudaMemcpyDeviceToDevice, ws.stream));
-            else {
-                CKS(ws.hq.ensure((size_t)R * ix->dim * 4));
-                memcpy(ws.hq.p, io.queries + (size_t)r0 * ix->dim, (size_t)R * ix->dim * 4);
-                CK(cudaMemcpyAsync(ws.Q.p, ws.hq.p, (size_t)R * ix->dim * 4, cudaMemcpyHostToDevice, ws.stream));
-            }
+static ProbeMode probe_mode(const pb_index *ix, const CallPlan &plan, int QS, bool tc) {
+    if (tc) return ProbeMode::TensorCore;
+    if (plan.all_eligible) return ProbeMode::AllEligible;
+    if (plan.big_probe) return ProbeMode::BigProbe;
+    // threshold-first selection needs the 16-bit table and at least n_probe chunk maxima
+    const int n = plan.n_probe;
+    int n_chunks = 0;
+    probe_chunk_rows(ix->K, n, &n_chunks);
+    const bool thr = plan.fast && !plan.d_elig && ix->probe16 && QS / 8 <= 32 && n_chunks >= n && n <= 192;
+    return thr ? ProbeMode::Threshold : ProbeMode::List;
+}
+
+// ---- H2D: the shape of the sub-batch at ps.b0, its query tokens and offsets ----
+static pb_status stage_h2d(pb_index *ix, Workspace &ws, const CallPlan &plan, Pass &ps) {
+    const SearchIO &io = *plan.io;
+    ps.B = (int)std::min<int64_t>(plan.QB, plan.Bt - ps.b0);
+    ps.r0 = io.q_off[ps.b0];
+    ps.R = io.q_off[ps.b0 + ps.B] - ps.r0;
+    for (int b = 0; b < ps.B; ++b) ps.nq_max = std::max(ps.nq_max, (int)(io.q_off[ps.b0 + b + 1] - io.q_off[ps.b0 + b]));
+    ps.QS = query_row_tokens(ps.nq_max);
+    const size_t qbytes = (size_t)ps.R * ix->dim * 4;
+    CKS(ws.Q.ensure(std::max<size_t>(qbytes, 16)));
+    CKS(ws.qoff.ensure((size_t)(ps.B + 1) * 4));
+    if (ps.R > 0) {
+        const float *src = io.queries + (size_t)ps.r0 * ix->dim;
+        if (io.queries_on_device) CK(cudaMemcpyAsync(ws.Q.p, src, qbytes, cudaMemcpyDeviceToDevice, ws.stream));
+        else {
+            CKS(ws.hq.ensure(qbytes));
+            memcpy(ws.hq.p, src, qbytes);
+            CK(cudaMemcpyAsync(ws.Q.p, ws.hq.p, qbytes, cudaMemcpyHostToDevice, ws.stream));
         }
-        CKS(ws.hcounts.ensure((size_t)(B + 1) * 4 + 16 + (size_t)(B + 2) * 8 + (size_t)B * 8 + (size_t)B * 7 * 4 + 192));
-        memcpy(ws.hcounts.p, qoff.data(), (size_t)(B + 1) * 4);
-        CK(cudaMemcpyAsync(ws.qoff.p, ws.hcounts.p, (size_t)(B + 1) * 4, cudaMemcpyHostToDevice, ws.stream));
-        if (prof) CK(cudaEventRecord(ws.ev[1], ws.stream));
+    }
+    CKS(ws.hcounts.ensure(PassHost().carve(nullptr, ps.B)));
+    ps.host.carve(ws.hcounts.as<char>(), ps.B);
+    for (int b = 0; b <= ps.B; ++b) ps.host.qoff[b] = (int)(io.q_off[ps.b0 + b] - ps.r0);
+    CK(cudaMemcpyAsync(ws.qoff.p, ps.host.qoff, (size_t)(ps.B + 1) * 4, cudaMemcpyHostToDevice, ws.stream));
+    return PB_OK;
+}
 
-        // ---- a2 centroid scores ----
-        if (!use_tc) CKS(ws.ST.ensure((size_t)B * ix->K * QS * sizeof(float)));
-        if (fast) {
-            CKS(ws.ST16.ensure((size_t)B * ix->K * QS * 2));
-            CKS(ws.qrange.ensure((size_t)B * 8 + 16));
-            CKS(ws.qflag.ensure((size_t)B * 4 + 16));
-            CKS(ws.qexp.ensure((size_t)B * 4 + 16));
-            CKS(ws.qnmax.ensure((size_t)B * 4 + 16));
-            k_query_range<<<B, 256, 0, ws.stream>>>(ws.Q.as<float>(), ws.qoff.as<int>(), ix->dim, ix->cmax,
-                                                    ws.qrange.as<float2>(), ws.qflag.as<int>(), ws.qexp.as<int>(),
-                                                    ws.qnmax.as<float>());
-            CK(cudaGetLastError());
-            L[PB_STAGE_CENTROID_SCORES] += 1;
-        }
-        const bool tc = use_tc;
-        int cells_cap = 0;
-        const int *d_probe_fallback = nullptr;  // device flag of the threshold-first probe (0 = it did the work)
-        bool probe_list_only = false;
-        if (tc) CKS(run_k1_tc(ix, ws, p, B, QS, nq_max, n_probe, batched, L, &cells_cap, &d_probe_fallback));
-        else CKS(launch_centroid_scores(ix, ws, B, QS, &L[PB_STAGE_CENTROID_SCORES], fast));
-        if (prof) CK(cudaEventRecord(ws.ev[2], ws.stream));
+// a2 + a3 on the tensor-core table.  Nothing is read back here: a flagged query or a probe-list overflow raises
+// ps.d_fallback on the device, the kernels after it stay memory-safe, and run_pass redoes the sub-batch on the exact
+// path once it sees the flag at the end.
+static pb_status run_k1_tc(pb_index *ix, Workspace &ws, const CallPlan &plan, Pass &ps) {
+    const pb_search_params *p = plan.p;
+    const int B = ps.B, QS = ps.QS, n = plan.n_probe;
+    int n_chunks = 0;
+    const int chunk_rows = probe_chunk_rows(ix->K, n, &n_chunks);
+    const int cm = 2 * ix->k1_margin + 1;
+    CKS(ws.Qi.ensure((size_t)B * QS * ix->dim * 4));
+    k_interleave_query_rows<<<dim3(8, B), 256, 0, ws.stream>>>(ws.Q.as<float>(), ws.qoff.as<int>(), QS, ix->dim, ws.Qi.as<float>());
+    CKS(launch_k1_table(ix, ws, B, QS, ws.ST16.as<unsigned short>(), ws.qflag.as<int>()));
+    g_stats.launches[PB_STAGE_CENTROID_SCORES] += 4;
+    const int cells_cap = (int)std::min<long long>((long long)QS * n, ix->K);
+    CKS(ws.sel.ensure((size_t)B * QS * n * 8));
+    CKS(ws.cells.ensure((size_t)B * cells_cap * 4));
+    CKS(ws.ncells.ensure((size_t)B * 4 + 16));
+    CKS(ws.ulist.ensure((size_t)B * cells_cap * 4));
+    CKS(ws.nulist.ensure((size_t)B * 4 + 16));
+    CKS(ws.k1rows.ensure((size_t)B * cells_cap * QS * 4));
+    CKS(launch_threshold_probe(ix, ws, B, QS, n, n_chunks, chunk_rows, true, &ps.d_fallback));
+    // the selected centroids, their exact rows, the variant's threshold rule
+    const int P = pow2_ceil(ps.nq_max * n);
+    CKS(set_smem(k_cells_unique, (size_t)P * 8));
+    k_cells_unique<<<B, 256, (size_t)P * 8, ws.stream>>>(ws.sel.as<u64>(), ws.qoff.as<int>(), QS, n, cells_cap,
+                                                         ws.ulist.as<uint32_t>(), ws.nulist.as<int>());
+    const size_t smr = (size_t)(PB_TOK_TILE * (ix->dim + 4) + PB_Q_TILE * ix->dim) * sizeof(float);
+    PB_DIM_SWITCH(ix->dim, {
+        auto kern = k_exact_rows<DIM>;
+        CKS(set_smem(kern, smr));
+        kern<<<dim3((cells_cap + PB_TOK_TILE - 1) / PB_TOK_TILE, B), 128, smr, ws.stream>>>(
+            ws.Qi.as<float>(), ws.qoff.as<int>(), QS, ix->centroids.as<float>(), ws.ulist.as<uint32_t>(), ws.nulist.as<int>(),
+            cells_cap, ws.k1rows.as<float>());
+    });
+    CKS(ws.cellflags.ensure((size_t)B * cells_cap * 4));
+    k_cells_thr<<<dim3(8, B), 256, 0, ws.stream>>>(
+        ws.sel.as<u64>(), ws.k1rows.as<float>(), ws.ulist.as<uint32_t>(), ws.nulist.as<int>(), ws.qoff.as<int>(), ix->K, QS, n,
+        cells_cap, p->has_centroid_score_threshold, p->centroid_score_threshold, plan.batched ? 1 : 0,
+        plan.batched ? (long long)p->centroid_batch_size : ix->K, ws.cellflags.as<int>(), ws.ST16.as<unsigned short>(),
+        ws.qrange.as<float2>(), cm, ws.Q.as<float>(), ix->centroids.as<float>(), ix->dim, ws.cmax16.as<unsigned short>(),
+        n_chunks, chunk_rows);
+    k_cells_emit<<<B, 256, 0, ws.stream>>>(ws.ulist.as<uint32_t>(), ws.nulist.as<int>(), ws.cellflags.as<int>(), cells_cap,
+                                           ws.cells.as<uint32_t>(), ws.ncells.as<int>());
+    CK(cudaGetLastError());
+    g_stats.launches[PB_STAGE_PROBE] += 4;
+    ps.cells_cap = cells_cap;
+    return PB_OK;
+}
 
-        // ---- a3 probe ----
-        if (tc) {
-            // cells are in place (run_k1_tc)
-        } else if (all_eligible) {
-            cells_cap = (int)n_elig;
-            CKS(ws.list.ensure((size_t)n_elig * 4 + 16));
-            CKS(ws.cells.ensure((size_t)B * cells_cap * 4));
+// ---- a2 centroid scores: the query range and flags, then the tensor-core table (with a3) or the fp32 one ----
+static pb_status stage_scores(pb_index *ix, Workspace &ws, const CallPlan &plan, Pass &ps) {
+    const int B = ps.B, QS = ps.QS;
+    if (!ps.tc) CKS(ws.ST.ensure((size_t)B * ix->K * QS * sizeof(float)));
+    if (plan.fast) {
+        CKS(ws.ST16.ensure((size_t)B * ix->K * QS * 2));
+        CKS(ws.qrange.ensure((size_t)B * 8 + 16));
+        CKS(ws.qflag.ensure((size_t)B * 4 + 16));
+        CKS(ws.qexp.ensure((size_t)B * 4 + 16));
+        CKS(ws.qnmax.ensure((size_t)B * 4 + 16));
+        k_query_range<<<B, 256, 0, ws.stream>>>(ws.Q.as<float>(), ws.qoff.as<int>(), ix->dim, ix->cmax,
+                                                ws.qrange.as<float2>(), ws.qflag.as<int>(), ws.qexp.as<int>(),
+                                                ws.qnmax.as<float>());
+        CK(cudaGetLastError());
+        g_stats.launches[PB_STAGE_CENTROID_SCORES] += 1;
+    }
+    if (ps.tc) return run_k1_tc(ix, ws, plan, ps);
+    return launch_centroid_scores(ix, ws, B, QS, &g_stats.launches[PB_STAGE_CENTROID_SCORES], plan.fast);
+}
+
+// a3 by per-lane lists: k_topn_partial scans the fp32 table, k_topn_merge keeps the top n per row, k_cells applies the
+// variant's threshold rule.  ProbeMode::Threshold runs the threshold-first probe first; the list scan then only does the
+// rows whose fallback flag is up.
+static pb_status probe_lists(pb_index *ix, Workspace &ws, const CallPlan &plan, Pass &ps) {
+    const pb_search_params *p = plan.p;
+    const int B = ps.B, QS = ps.QS, n = plan.n_probe;
+    const int n_chunks = (int)((ix->K + 1023) / 1024);
+    ps.cells_cap = (int)std::min<long long>((long long)QS * n, ix->K);
+    CKS(ws.partial.ensure((size_t)B * QS * n_chunks * n * 8));
+    CKS(ws.sel.ensure((size_t)B * QS * n * 8));
+    CKS(ws.cells.ensure((size_t)B * ps.cells_cap * 4));
+    CKS(ws.ncells.ensure((size_t)B * 4 + 16));
+    size_t sm1 = (size_t)4 * n * 32 * 8;
+    CKS(set_smem(k_topn_partial, sm1));
+    const bool thr = ps.probe == ProbeMode::Threshold;
+    int t_chunks = 0;
+    const int t_rows = probe_chunk_rows(ix->K, n, &t_chunks);
+    if (thr) CKS(launch_threshold_probe(ix, ws, B, QS, n, t_chunks, t_rows, false, &ps.d_fallback));
+    k_topn_partial<<<dim3((n_chunks + 3) / 4, B, (QS + 31) / 32), 128, sm1, ws.stream>>>(
+        ws.ST.as<float>(), ws.qoff.as<int>(), ix->K, QS, n, plan.d_elig, ws.partial.as<u64>(), n_chunks, ps.d_fallback, 1);
+    k_topn_merge<<<dim3(QS, B), 32, 0, ws.stream>>>(ws.partial.as<u64>(), ws.qoff.as<int>(), QS, n, n_chunks,
+                                                  ws.sel.as<u64>(), ps.d_fallback, 1);
+    const int P = pow2_ceil(ps.nq_max * n);
+    size_t sm2 = (size_t)P * 12;
+    CKS(set_smem(k_cells, sm2));
+    k_cells<<<B, 256, sm2, ws.stream>>>(ws.sel.as<u64>(), ws.ST.as<float>(), ws.qoff.as<int>(), ix->K, QS, n,
+                                        ps.cells_cap, p->has_centroid_score_threshold, p->centroid_score_threshold,
+                                        plan.batched ? 1 : 0, plan.batched ? (long long)p->centroid_batch_size : ix->K,
+                                        ws.cells.as<uint32_t>(), ws.ncells.as<int>(),
+                                        thr ? ws.cmax16.as<unsigned short>() : nullptr, t_chunks, t_rows,
+                                        ws.qrange.as<float2>(), ps.d_fallback);
+    CK(cudaGetLastError());
+    g_stats.launches[PB_STAGE_PROBE] += 3;
+    return PB_OK;
+}
+
+// ---- a3 probe: the cells (centroids) each query reads ----
+static pb_status stage_probe(pb_index *ix, Workspace &ws, const CallPlan &plan, Pass &ps) {
+    const pb_search_params *p = plan.p;
+    const int B = ps.B, QS = ps.QS;
+    switch (ps.probe) {
+        case ProbeMode::TensorCore: return PB_OK;  // the cells are in place (run_k1_tc)
+        case ProbeMode::Threshold:
+        case ProbeMode::List: return probe_lists(ix, ws, plan, ps);
+        case ProbeMode::AllEligible: {
+            ps.cells_cap = (int)plan.n_elig;
+            CKS(ws.list.ensure((size_t)plan.n_elig * 4 + 16));
+            CKS(ws.cells.ensure((size_t)B * ps.cells_cap * 4));
             CKS(ws.ncells.ensure((size_t)B * 4 + 16));
             int *d_listn = reinterpret_cast<int *>(ws.misc.as<char>() + 16);
-            k_cells_from_bits<<<1, 1024, 0, ws.stream>>>(d_elig, ix->K, ws.list.as<uint32_t>(), d_listn);
+            k_cells_from_bits<<<1, 1024, 0, ws.stream>>>(plan.d_elig, ix->K, ws.list.as<uint32_t>(), d_listn);
             k_cells_filter_list<<<B, 256, 0, ws.stream>>>(ws.list.as<uint32_t>(), d_listn, ws.ST.as<float>(),
                                                           ws.qoff.as<int>(), ix->K, QS, p->has_centroid_score_threshold,
-                                                          p->centroid_score_threshold, cells_cap, ws.cells.as<uint32_t>(),
+                                                          p->centroid_score_threshold, ps.cells_cap, ws.cells.as<uint32_t>(),
                                                           ws.ncells.as<int>());
-            CK(cudaGetLastError());
-            L[PB_STAGE_PROBE] += 2;
-        } else if (big_probe) {
-            cells_cap = (int)std::min<long long>((long long)QS * n_probe, ix->K);
-            CKS(ws.cellbits.ensure((size_t)B * Wk * 4));
-            CKS(ws.cells.ensure((size_t)B * cells_cap * 4));
+            break;
+        }
+        case ProbeMode::BigProbe: {
+            ps.cells_cap = (int)std::min<long long>((long long)QS * plan.n_probe, ix->K);
+            CKS(ws.cellbits.ensure((size_t)B * plan.Wk * 4));
+            CKS(ws.cells.ensure((size_t)B * ps.cells_cap * 4));
             CKS(ws.ncells.ensure((size_t)B * 4 + 16));
-            k_topn_select_row<<<dim3(QS, B), 256, 0, ws.stream>>>(ws.ST.as<float>(), ws.qoff.as<int>(), ix->K, QS, n_probe,
-                                                                  d_elig, ws.cellbits.as<uint32_t>(), Wk);
-            k_cells_from_query_bits<<<B, 1024, 0, ws.stream>>>(ws.cellbits.as<uint32_t>(), Wk, ws.ST.as<float>(),
+            k_topn_select_row<<<dim3(QS, B), 256, 0, ws.stream>>>(ws.ST.as<float>(), ws.qoff.as<int>(), ix->K, QS, plan.n_probe,
+                                                                  plan.d_elig, ws.cellbits.as<uint32_t>(), plan.Wk);
+            k_cells_from_query_bits<<<B, 1024, 0, ws.stream>>>(ws.cellbits.as<uint32_t>(), plan.Wk, ws.ST.as<float>(),
                                                                ws.qoff.as<int>(), ix->K, QS, p->has_centroid_score_threshold,
-                                                               p->centroid_score_threshold, cells_cap, ws.cells.as<uint32_t>(),
+                                                               p->centroid_score_threshold, ps.cells_cap, ws.cells.as<uint32_t>(),
                                                                ws.ncells.as<int>());
-            CK(cudaGetLastError());
-            L[PB_STAGE_PROBE] += 2;
-        } else {
-            const int n = n_probe;
-            const int n_chunks = (int)((ix->K + 1023) / 1024);
-            cells_cap = (int)std::min<long long>((long long)QS * n, ix->K);
-            CKS(ws.partial.ensure((size_t)B * QS * n_chunks * n * 8));
-            CKS(ws.sel.ensure((size_t)B * QS * n * 8));
-            CKS(ws.cells.ensure((size_t)B * cells_cap * 4));
-            CKS(ws.ncells.ensure((size_t)B * 4 + 16));
-            size_t sm1 = (size_t)4 * n * 32 * 8;
-            CKS(set_smem(k_topn_partial, sm1));
-            // threshold-first selection on the 16-bit table when there is one (k_chunkmax16 / k_collect16);
-            // the per-lane list scan of k_topn_partial otherwise, or when the device raises `fallback`
-            const int GQ = QS / 8;
-            int t_chunks = 0;
-            const int t_rows = probe_chunk_rows(ix->K, n, &t_chunks);
-            const bool thr_path = fast && !d_elig && ix->probe16 && GQ <= 32 && t_chunks >= n && n <= 192;
-            int *d_fallback = nullptr;
-            probe_list_only = !thr_path;
-            if (thr_path) {
-                const int cap = n * std::max(2, 128 / n);
-                CKS(ws.cmax16.ensure((size_t)B * t_chunks * QS * 2));
-                CKS(ws.tau16.ensure((size_t)B * QS * 4));
-                CKS(ws.plist.ensure((size_t)B * QS * cap * 8));
-                CKS(ws.pcount.ensure((size_t)B * QS * 4 + 16));
-                CK(cudaMemsetAsync(ws.plist.p, 0, (size_t)B * QS * cap * 8, ws.stream));
-                CK(cudaMemsetAsync(ws.pcount.p, 0, (size_t)B * QS * 4 + 16, ws.stream));
-                d_fallback = ws.pcount.as<int>() + (size_t)B * QS;
-                d_probe_fallback = d_fallback;
-                k_chunkmax16<<<dim3((t_chunks + 3) / 4, B), 128, 0, ws.stream>>>(ws.ST16.as<unsigned short>(), ix->K, QS, t_chunks,
-                                                                                 t_rows, ws.cmax16.as<unsigned short>());
-                k_tau16<<<dim3(QS, B), 32, 0, ws.stream>>>(ws.cmax16.as<unsigned short>(), ws.qoff.as<int>(), QS, n, t_chunks,
-                                                          ws.qflag.as<int>(), ws.tau16.as<uint32_t>(), d_fallback);
-                k_collect16<<<dim3((t_chunks + 3) / 4, B), 128, 0, ws.stream>>>(
-                    ws.ST16.as<unsigned short>(), ws.ST.as<float>(), ix->K, QS, t_chunks, t_rows, ws.tau16.as<uint32_t>(), cap,
-                    ws.pcount.as<int>(), ws.plist.as<u64>(), d_fallback);
-                k_topn_merge<<<dim3(QS, B), 32, 0, ws.stream>>>(ws.plist.as<u64>(), ws.qoff.as<int>(), QS, n, cap / n,
-                                                              ws.sel.as<u64>(), d_fallback, 0);
-                CK(cudaGetLastError());
-                L[PB_STAGE_PROBE] += 4;
-            }
-            k_topn_partial<<<dim3((n_chunks + 3) / 4, B, (QS + 31) / 32), 128, sm1, ws.stream>>>(
-                ws.ST.as<float>(), ws.qoff.as<int>(), ix->K, QS, n, d_elig, ws.partial.as<u64>(), n_chunks, d_fallback, 1);
-            k_topn_merge<<<dim3(QS, B), 32, 0, ws.stream>>>(ws.partial.as<u64>(), ws.qoff.as<int>(), QS, n, n_chunks,
-                                                          ws.sel.as<u64>(), d_fallback, 1);
-            int P = 1;
-            while (P < std::max(nq_max * n, 1)) P <<= 1;
-            size_t sm2 = (size_t)P * 12;
-            CKS(set_smem(k_cells, sm2));
-            k_cells<<<B, 256, sm2, ws.stream>>>(ws.sel.as<u64>(), ws.ST.as<float>(), ws.qoff.as<int>(), ix->K, QS, n,
-                                                cells_cap, p->has_centroid_score_threshold, p->centroid_score_threshold,
-                                                batched ? 1 : 0, batched ? (long long)p->centroid_batch_size : ix->K,
-                                                ws.cells.as<uint32_t>(), ws.ncells.as<int>(),
-                                                thr_path ? ws.cmax16.as<unsigned short>() : nullptr, t_chunks, t_rows,
-                                                ws.qrange.as<float2>(), d_fallback);
-            CK(cudaGetLastError());
-            L[PB_STAGE_PROBE] += 3;
+            break;
         }
-        if (prof) CK(cudaEventRecord(ws.ev[3], ws.stream));
+    }
+    CK(cudaGetLastError());
+    g_stats.launches[PB_STAGE_PROBE] += 2;
+    return PB_OK;
+}
 
-        // ---- a4 candidates ----
-        CKS(ws.bitmap.ensure((size_t)B * Wd * 4));
-        CKS(ws.cand.ensure((size_t)B * ix->D * 4));
-        CKS(ws.ncand.ensure((size_t)B * 4 + 16));
-        k_mark<<<dim3(cells_cap, B), 128, 0, ws.stream>>>(ws.cells.as<uint32_t>(), ws.ncells.as<int>(), cells_cap,
-                                                         ix->ivf.as<uint32_t>(), ix->ivf_off.as<long long>(), d_subset_bits,
+// ---- a4 candidates: the docs of the cells' posting lists, once each ----
+static pb_status stage_candidates(pb_index *ix, Workspace &ws, const CallPlan &plan, Pass &ps) {
+    const int B = ps.B;
+    const long long Wd = plan.Wd;
+    CKS(ws.bitmap.ensure((size_t)B * Wd * 4));
+    CKS(ws.cand.ensure((size_t)B * ix->D * 4));
+    CKS(ws.ncand.ensure((size_t)B * 4 + 16));
+    k_mark<<<dim3(ps.cells_cap, B), 128, 0, ws.stream>>>(ws.cells.as<uint32_t>(), ws.ncells.as<int>(), ps.cells_cap,
+                                                         ix->ivf.as<uint32_t>(), ix->ivf_off.as<long long>(), plan.d_subset_bits,
                                                          ws.bitmap.as<uint32_t>(), Wd);
-        const int slices = (int)std::max<long long>(1, std::min<long long>(32, (4ll * ix->sm_count + B - 1) / B));
-        CKS(ws.slicecnt.ensure((size_t)B * slices * 4));
-        k_compact_count<<<dim3(slices, B), 256, 0, ws.stream>>>(ws.bitmap.as<uint32_t>(), Wd, ws.slicecnt.as<int>());
-        k_compact_emit<<<dim3(slices, B), 256, 0, ws.stream>>>(ws.bitmap.as<uint32_t>(), Wd, ws.slicecnt.as<int>(),
-                                                               ws.cand.as<uint32_t>(), ix->D, ws.ncand.as<int>());
-        CK(cudaGetLastError());
-        L[PB_STAGE_CANDIDATES] += 3;
-        if (prof) CK(cudaEventRecord(ws.ev[4], ws.stream));
+    const int slices = (int)std::max<long long>(1, std::min<long long>(32, (4ll * ix->sm_count + B - 1) / B));
+    CKS(ws.slicecnt.ensure((size_t)B * slices * 4));
+    k_compact_count<<<dim3(slices, B), 256, 0, ws.stream>>>(ws.bitmap.as<uint32_t>(), Wd, ws.slicecnt.as<int>());
+    k_compact_emit<<<dim3(slices, B), 256, 0, ws.stream>>>(ws.bitmap.as<uint32_t>(), Wd, ws.slicecnt.as<int>(),
+                                                           ws.cand.as<uint32_t>(), ix->D, ws.ncand.as<int>());
+    CK(cudaGetLastError());
+    g_stats.launches[PB_STAGE_CANDIDATES] += 3;
+    return PB_OK;
+}
 
-        // ---- a5 approximate scores ----
-        CKS(ws.counters.ensure((size_t)(B + 2) * 8));  // [0] candidate codes gathered, [1+b] kept-doc tokens, [B+1] re-check gathers
-        CK(cudaMemsetAsync(ws.counters.p, 0, (size_t)(B + 2) * 8, ws.stream));
-        CKS(ws.approx.ensure((size_t)B * ix->D * 4));
-        CKS(ws.keys.ensure((size_t)B * ix->D * 8));
-        const uint32_t *cand_list = ws.cand.as<uint32_t>();
-        const int *cand_n = ws.ncand.as<int>();
-        if (fast) {
-            CKS(ws.lsum.ensure((size_t)B * ix->D * 4));
-            CKS(ws.cand2.ensure((size_t)B * ix->D * 4));
-            CKS(ws.ncand2.ensure((size_t)B * 4 + 16));
-            const dim3 ga(ix->sm_count * ix->approx_grid, B);
-            const unsigned short *st16 = ws.ST16.as<unsigned short>();
-            const uint32_t *list = ws.cand.as<uint32_t>();
-            const int *list_n = ws.ncand.as<int>();
-            unsigned long long *cnt = ws.counters.as<unsigned long long>();
-            KEV_BEGIN(PB_KERNEL_APPROX16);
-            (QS <= 32 ? k_approx16<4> : k_approx16<8>)<<<ga, 256, 0, ws.stream>>>(
-                st16, ws.qoff.as<int>(), ix->K, QS, ix->ucodes.as<uint32_t>(), ix->udoc_off.as<long long>(), list, ix->D, list_n,
-                ws.lsum.as<uint32_t>(), cnt);
-            KEV_END(PB_KERNEL_APPROX16);
-            // band per query token in code units (W = band * nq + 8).  Exact table: +-1 code of rounding per token and side
-            // plus the fp32 summation error -> 4.  Estimate table (k_scores_tc.cuh): W = nq (1.004 + 2 err) + nq^2/256 + 4
-            // <= nq (ceil(1.004 + 2 err) + 1) + 8 for nq <= 256.
-            const int band_per_q = tc ? (int)ceilf(1.004f + 2.0f * std::max(k1_err_codes(ix->dim), (float)(ix->k1_margin - 1))) + 1 : 4;
-            k_select_u32<<<B, 1024, 0, ws.stream>>>(ws.lsum.as<uint32_t>(), list_n, M, band_per_q, ws.lsum.as<uint32_t>(), list,
-                                                    list_n, ix->D, ws.qoff.as<int>(), ws.qflag.as<int>(),
-                                                    ws.cand2.as<uint32_t>(), ws.ncand2.as<int>());
-            CK(cudaGetLastError());
-            L[PB_STAGE_APPROX] += 2;
-            cand_list = ws.cand2.as<uint32_t>();
-            cand_n = ws.ncand2.as<int>();
-        }
-        if (tc) {  // the exact approximate score of the docs around the cut from pinned-order dots (no dense fp32 S)
-            const int rc_cap = 2 * Mcap + 1024, pair_cap = 64 * rc_cap;
-            CKS(ws.rcmax.ensure((size_t)B * rc_cap * QS * 4));
-            CKS(ws.rcpairs.ensure((size_t)B * pair_cap * 8));
-            CKS(ws.rcn.ensure((size_t)B * 4 + 16));
-            CK(cudaMemsetAsync(ws.rcn.p, 0, (size_t)B * 4, ws.stream));
-            int *d_fb = const_cast<int *>(d_probe_fallback);
-            (QS <= 32 ? k_recheck_pairs<4> : k_recheck_pairs<8>)<<<dim3(ix->sm_count * 2, B), 256, 0, ws.stream>>>(
-                ws.ST16.as<unsigned short>(), ws.qoff.as<int>(), ix->K, QS, ix->ucodes.as<uint32_t>(), ix->udoc_off.as<long long>(),
-                cand_list, ix->D, cand_n, 2 * ix->k1_margin + 1, rc_cap, pair_cap, ws.rcpairs.as<u64>(), ws.rcn.as<int>(), d_fb,
-                ws.counters.as<unsigned long long>() + B + 1);
-            k_recheck_dots<<<dim3(ix->sm_count * 2, B), 128, 0, ws.stream>>>(ws.rcpairs.as<u64>(), ws.rcn.as<int>(), pair_cap,
-                                                                             ws.Q.as<float>(), ws.qoff.as<int>(),
-                                                                             ix->centroids.as<float>(), ix->dim, rc_cap, QS,
-                                                                             ws.rcmax.as<uint32_t>());
-            k_recheck_sum<<<dim3(ix->sm_count, B), 256, 0, ws.stream>>>(ws.rcmax.as<uint32_t>(), ws.qoff.as<int>(), QS, cand_list,
-                                                                        ix->D, cand_n, rc_cap, ws.approx.as<float>(),
-                                                                        ws.keys.as<u64>(), (uint32_t)ix->doc_id_base);
-            L[PB_STAGE_APPROX] += 2;
-        }
-        else
-            k_approx<<<dim3(ix->sm_count * 8, B), 256, 0, ws.stream>>>(
-                ws.ST.as<float>(), ws.qoff.as<int>(), ix->K, QS, ix->ucodes.as<uint32_t>(), ix->udoc_off.as<long long>(),
-                cand_list, ix->D, cand_n, ws.approx.as<float>(), ws.keys.as<u64>(),
-                fast ? ws.counters.as<unsigned long long>() + B + 1 : ws.counters.as<unsigned long long>(),
-                (uint32_t)ix->doc_id_base);
+// ---- a5 approximate scores: the two-pass approximate stage (with the re-check on the tensor-core path), or k_approx ----
+static pb_status stage_approx(pb_index *ix, Workspace &ws, const CallPlan &plan, Pass &ps) {
+    const int B = ps.B, QS = ps.QS;
+    int *L = g_stats.launches;
+    CKS(ws.counters.ensure((size_t)(B + 2) * 8));  // [0] candidate codes gathered, [1+b] kept-doc tokens, [B+1] re-check gathers
+    CK(cudaMemsetAsync(ws.counters.p, 0, (size_t)(B + 2) * 8, ws.stream));
+    CKS(ws.approx.ensure((size_t)B * ix->D * 4));
+    CKS(ws.keys.ensure((size_t)B * ix->D * 8));
+    ps.cand_list = ws.cand.as<uint32_t>();
+    ps.cand_n = ws.ncand.as<int>();
+    if (plan.fast) {
+        CKS(ws.lsum.ensure((size_t)B * ix->D * 4));
+        CKS(ws.cand2.ensure((size_t)B * ix->D * 4));
+        CKS(ws.ncand2.ensure((size_t)B * 4 + 16));
+        const dim3 ga(ix->sm_count * ix->approx_grid, B);
+        const uint32_t *list = ws.cand.as<uint32_t>();
+        const int *list_n = ws.ncand.as<int>();
+        KEV_BEGIN(PB_KERNEL_APPROX16);
+        (QS <= 32 ? k_approx16<4> : k_approx16<8>)<<<ga, 256, 0, ws.stream>>>(
+            ws.ST16.as<unsigned short>(), ws.qoff.as<int>(), ix->K, QS, ix->ucodes.as<uint32_t>(), ix->udoc_off.as<long long>(),
+            list, ix->D, list_n, ws.lsum.as<uint32_t>(), ws.counters.as<unsigned long long>());
+        KEV_END(PB_KERNEL_APPROX16);
+        // band per query token in code units (W = band * nq + 8).  Exact table: +-1 code of rounding per token and side
+        // plus the fp32 summation error -> 4.  Estimate table (k_scores_tc.cuh): W = nq (1.004 + 2 err) + nq^2/256 + 4
+        // <= nq (ceil(1.004 + 2 err) + 1) + 8 for nq <= 256.
+        const int band_per_q = ps.tc ? (int)ceilf(1.004f + 2.0f * std::max(k1_err_codes(ix->dim), (float)(ix->k1_margin - 1))) + 1 : 4;
+        k_select_u32<<<B, 1024, 0, ws.stream>>>(ws.lsum.as<uint32_t>(), list_n, plan.M, band_per_q, ws.lsum.as<uint32_t>(), list,
+                                                list_n, ix->D, ws.qoff.as<int>(), ws.qflag.as<int>(),
+                                                ws.cand2.as<uint32_t>(), ws.ncand2.as<int>());
         CK(cudaGetLastError());
-        L[PB_STAGE_APPROX] += 1;
-        if (prof) CK(cudaEventRecord(ws.ev[5], ws.stream));
-        if (vote) {
-            // The probe flags are the same on every rank (a2/a3 are replicated), a re-check overflow is not: it depends
-            // on this shard's documents.  Nor is the path: a rank without tensor-core operands (a shard with no tokens)
-            // or with other settings runs the exact pass and votes 0.  Every rank's flag word is gathered here, before
-            // exchange 1, and the pass is abandoned on all ranks if any rank raised it; a lone redo would pair its
-            // exchanges with the peers' next ones.  The kernels so far have restored their scratch invariants
-            // (bitmaps, re-check maxima).
-            const u64 *all = nullptr;
-            CKS(shard_vote(ix, ws, 0, tc ? d_probe_fallback : nullptr, &all));
-            u64 any = 0;
-            for (int g = 0; g < ix->world; ++g) any |= all[g];
-            if (any) {
-                *redo = true;
-                return PB_OK;
-            }
-        }
+        L[PB_STAGE_APPROX] += 2;
+        ps.cand_list = ws.cand2.as<uint32_t>();
+        ps.cand_n = ws.ncand2.as<int>();
+    }
+    if (ps.tc) {  // the exact approximate score of the docs around the cut from pinned-order dots (no dense fp32 S)
+        const int rc_cap = 2 * plan.Mcap + 1024, pair_cap = 64 * rc_cap;
+        CKS(ws.rcmax.ensure((size_t)B * rc_cap * QS * 4));
+        CKS(ws.rcpairs.ensure((size_t)B * pair_cap * 8));
+        CKS(ws.rcn.ensure((size_t)B * 4 + 16));
+        CK(cudaMemsetAsync(ws.rcn.p, 0, (size_t)B * 4, ws.stream));
+        (QS <= 32 ? k_recheck_pairs<4> : k_recheck_pairs<8>)<<<dim3(ix->sm_count * 2, B), 256, 0, ws.stream>>>(
+            ws.ST16.as<unsigned short>(), ws.qoff.as<int>(), ix->K, QS, ix->ucodes.as<uint32_t>(), ix->udoc_off.as<long long>(),
+            ps.cand_list, ix->D, ps.cand_n, 2 * ix->k1_margin + 1, rc_cap, pair_cap, ws.rcpairs.as<u64>(), ws.rcn.as<int>(),
+            ps.d_fallback, ws.counters.as<unsigned long long>() + B + 1);
+        k_recheck_dots<<<dim3(ix->sm_count * 2, B), 128, 0, ws.stream>>>(ws.rcpairs.as<u64>(), ws.rcn.as<int>(), pair_cap,
+                                                                         ws.Q.as<float>(), ws.qoff.as<int>(),
+                                                                         ix->centroids.as<float>(), ix->dim, rc_cap, QS,
+                                                                         ws.rcmax.as<uint32_t>());
+        k_recheck_sum<<<dim3(ix->sm_count, B), 256, 0, ws.stream>>>(ws.rcmax.as<uint32_t>(), ws.qoff.as<int>(), QS, ps.cand_list,
+                                                                    ix->D, ps.cand_n, rc_cap, ws.approx.as<float>(),
+                                                                    ws.keys.as<u64>(), (uint32_t)ix->doc_id_base);
+        L[PB_STAGE_APPROX] += 2;
+    } else
+        k_approx<<<dim3(ix->sm_count * 8, B), 256, 0, ws.stream>>>(
+            ws.ST.as<float>(), ws.qoff.as<int>(), ix->K, QS, ix->ucodes.as<uint32_t>(), ix->udoc_off.as<long long>(),
+            ps.cand_list, ix->D, ps.cand_n, ws.approx.as<float>(), ws.keys.as<u64>(),
+            plan.fast ? ws.counters.as<unsigned long long>() + B + 1 : ws.counters.as<unsigned long long>(),
+            (uint32_t)ix->doc_id_base);
+    CK(cudaGetLastError());
+    L[PB_STAGE_APPROX] += 1;
+    return PB_OK;
+}
 
-        // ---- a6 cut ----
-        CKS(ws.kept.ensure((size_t)B * Mcap * 4));
-        CKS(ws.nkept.ensure((size_t)B * 4 + 16));
-        CKS(ws.tokp.ensure((size_t)B * (Mcap + 1) * 8));
-        if (sharded) CKS(ws.lkeys.ensure((size_t)B * Mcap * 8));
-        int Pm = 1;
-        while (Pm < Mcap) Pm <<= 1;
-        CKS(set_smem(k_cut, (size_t)Pm * 8));
-        k_cut<<<B, 1024, (size_t)Pm * 8, ws.stream>>>(ws.keys.as<u64>(), ws.approx.as<float>(), ix->D, cand_n, M,
-                                                      Mcap, ix->doc_off.as<long long>(), ws.kept.as<uint32_t>(),
-                                                      ws.nkept.as<int>(), ws.tokp.as<long long>(),
-                                                      ws.counters.as<long long>() + 1, (uint32_t)ix->doc_id_base,
-                                                      sharded ? ws.lkeys.as<u64>() : nullptr);
+// ---- a6 cut: the top M per query by approximate score; sharded, exchange 1 turns it into this shard's share of the
+// global cut ----
+static pb_status stage_cut(pb_index *ix, Workspace &ws, const CallPlan &plan, Pass &ps) {
+    const int B = ps.B, M = plan.M, Mcap = plan.Mcap;
+    const bool sharded = plan.sharded;
+    CKS(ws.kept.ensure((size_t)B * Mcap * 4));
+    CKS(ws.nkept.ensure((size_t)B * 4 + 16));
+    CKS(ws.tokp.ensure((size_t)B * (Mcap + 1) * 8));
+    if (sharded) CKS(ws.lkeys.ensure((size_t)B * Mcap * 8));
+    const int Pm = pow2_ceil(Mcap);
+    CKS(set_smem(k_cut, (size_t)Pm * 8));
+    k_cut<<<B, 1024, (size_t)Pm * 8, ws.stream>>>(ws.keys.as<u64>(), ws.approx.as<float>(), ix->D, ps.cand_n, M,
+                                                  Mcap, ix->doc_off.as<long long>(), ws.kept.as<uint32_t>(),
+                                                  ws.nkept.as<int>(), ws.tokp.as<long long>(),
+                                                  ws.counters.as<long long>() + 1, (uint32_t)ix->doc_id_base,
+                                                  sharded ? ws.lkeys.as<u64>() : nullptr);
+    CK(cudaGetLastError());
+    g_stats.launches[PB_STAGE_CUT] += 1;
+    if (sharded) {
+        // exchange 1: every shard's sorted top-M cut keys -> global cut -> my members (SURVEY 8e)
+        const int G = ix->world;
+        CKS(ws.gkeys.ensure((size_t)G * B * M * 8));
+        CKS(ws.krank.ensure((size_t)B * Mcap * 4));
+        CKS(shard_allgather(ix, ws.stream, ws.lkeys.p, ws.gkeys.p, (size_t)B * M));
+        k_merge_cut<<<B, 1024, 0, ws.stream>>>(ws.gkeys.as<u64>(), G, ix->rank, B, M, (uint32_t)ix->doc_id_base, ix->D,
+                                               ix->doc_off.as<long long>(), ws.kept.as<uint32_t>(),
+                                               ws.krank.as<uint32_t>(), ws.nkept.as<int>(),
+                                               ws.tokp.as<long long>(), ws.counters.as<long long>() + 1);
         CK(cudaGetLastError());
-        L[PB_STAGE_CUT] += 1;
-        if (sharded) {
-            // exchange 1: every shard's sorted top-M cut keys -> global cut -> my members (SURVEY 8e)
-            const int G = ix->world;
-            CKS(ws.gkeys.ensure((size_t)G * B * M * 8));
-            CKS(ws.krank.ensure((size_t)B * Mcap * 4));
-            CKS(shard_allgather(ix, ws.stream, ws.lkeys.p, ws.gkeys.p, (size_t)B * M));
-            k_merge_cut<<<B, 1024, 0, ws.stream>>>(ws.gkeys.as<u64>(), G, ix->rank, B, M, (uint32_t)ix->doc_id_base, ix->D,
-                                                   ix->doc_off.as<long long>(), ws.kept.as<uint32_t>(),
-                                                   ws.krank.as<uint32_t>(), ws.nkept.as<int>(),
-                                                   ws.tokp.as<long long>(), ws.counters.as<long long>() + 1);
-            CK(cudaGetLastError());
-            L[PB_STAGE_CUT] += 2;
-        }
-        if (prof) CK(cudaEventRecord(ws.ev[6], ws.stream));
+        g_stats.launches[PB_STAGE_CUT] += 2;
+    }
+    ps.kv = KeptView{ws.kept.as<uint32_t>(), ws.nkept.as<int>(), ws.tokp.as<long long>(),
+                     sharded ? ws.krank.as<uint32_t>() : nullptr};
+    return PB_OK;
+}
 
-        // ---- a7+a8 exact ----
-        CKS(ws.maxkey.ensure((size_t)B * Mcap * QS * 4));
-        CKS(ws.exact.ensure((size_t)B * Mcap * 4));
-        CKS(ws.fkeys.ensure((size_t)B * Mcap * 8));
-        KeptView kv{ws.kept.as<uint32_t>(), ws.nkept.as<int>(), ws.tokp.as<long long>(),
-                    sharded ? ws.krank.as<uint32_t>() : nullptr};
-        // only the top_k need exact scores: the tensor-core filter drops the docs that provably cannot reach them
-        // the linear form needs the 16-bit score table of this pass (a flagged query publishes no estimate and keeps
-        // every doc); without a table (PB_FAST_APPROX=0) the decompressing form estimates from fp16 centroids
-        const bool linear = fast && !ix->filter_v1 && ix->tok_inv_norm.p;
-        const float eps_unit = linear ? filter_eps_unit2(ix, tc ? ix->k1_margin : 0) : filter_eps_unit(ix);
-        const bool filt = ix->fast_exact && !io.trace && ix->centroids_f16.p && eps_unit > 0.0f && nq_max <= 64 &&
-                          top_k < Mcap && ix->packed % 4 == 0;
-        bool pairs = false;
-        if (filt) {
-            CKS(ws.est.ensure((size_t)B * Mcap * 4));
-            CKS(ws.kept2.ensure((size_t)B * Mcap * 4));
-            CKS(ws.krank2.ensure((size_t)B * Mcap * 4));
-            CKS(ws.nkept2.ensure((size_t)B * 4 + 16));
-            CKS(ws.tokp2.ensure((size_t)B * (Mcap + 1) * 8));
-            CKS(ws.ktok2.ensure((size_t)B * 8 + 16));
-            if (!fast) {  // the two-pass mode computed it with the score range
-                CKS(ws.qnmax.ensure((size_t)B * 4 + 16));
-                k_query_range<<<B, 256, 0, ws.stream>>>(ws.Q.as<float>(), ws.qoff.as<int>(), ix->dim, ix->cmax, nullptr, nullptr,
-                                                        nullptr, ws.qnmax.as<float>());
-                CK(cudaGetLastError());
-                L[PB_STAGE_EXACT] += 1;
-            }
-            KeptView kv2{ws.kept2.as<uint32_t>(), ws.nkept2.as<int>(), ws.tokp2.as<long long>(), ws.krank2.as<uint32_t>()};
-            // pair form of the exact stage: pass 2 of the estimate over the survivors lists the (token, q) pairs that can
-            // hold a per-token maximum, k_pair_exact evaluates them in the pinned order; a query whose list overflows
-            // (or that published no estimate) goes through k_exact
-            pairs = linear && ix->pair_exact && Mcap <= 65535 && QS <= 256;
-            if (pairs) {
-                CKS(ws.estkey.ensure((size_t)B * Mcap * QS * 4));
-                CKS(ws.srcrank.ensure((size_t)B * Mcap * 4));
-            }
-            CKS(launch_filter(ix, ws, kv, kv2, B, QS, Mcap, top_k, (long long)Mcap * std::max(ix->max_doclen, 1), eps_unit,
-                              nq_max, linear, pairs, &L[PB_STAGE_EXACT]));
-            kv = kv2;
-            if (!sharded) kv.krank = nullptr;  // survivors keep their order, so position breaks ties the same way
+// a8 in pair form: pass 2 of the estimate over the filter's survivors lists the (token, q) pairs that can hold a
+// per-token maximum, k_pair_exact evaluates them in the pinned order; a query whose list overflows (or that published
+// no estimate) goes through k_exact
+static pb_status launch_pair_exact(pb_index *ix, Workspace &ws, const CallPlan &plan, const Pass &ps, float eps_unit) {
+    const int B = ps.B, QS = ps.QS, Mcap = plan.Mcap;
+    const long long max_tokens = (long long)Mcap * std::max(ix->max_doclen, 1);
+    const int pair_cap = 16 * Mcap + 4096;  // ~ (top_k + ties) * nq * (1 + a few) pairs per query in practice
+    CKS(ws.xpairs.ensure((size_t)B * pair_cap * 8));
+    CKS(ws.xnpairs.ensure((size_t)B * 4 + 16));
+    CKS(ws.needexact.ensure((size_t)B * 4 + 16));
+    CK(cudaMemsetAsync(ws.xnpairs.p, 0, (size_t)B * 4, ws.stream));
+    KEV_BEGIN(PB_KERNEL_EXACT);  // pass 2 + pair evaluation + the (normally empty) k_exact of flagged queries
+    CKS(launch_maxsim_tc(ix, ws, ps.kv, B, QS, Mcap, max_tokens, ps.nq_max, ws.estkey.as<uint32_t>(),
+                         ws.srcrank.as<uint32_t>(), eps_unit, ws.xpairs.as<u64>(), ws.xnpairs.as<int>(), pair_cap, -1));
+    k_pair_overflow<<<(B + 255) / 256, 256, 0, ws.stream>>>(ws.xnpairs.as<int>(), pair_cap, ws.qflag.as<int>(), B,
+                                                            ws.needexact.as<int>());
+    CK(cudaGetLastError());
+    const size_t smp = ((size_t)(ps.nq_max + 256) * (ix->dim + 1) + 256) * 4;
+    const int pe_ctas = std::max(1, std::min(16, (2 * ix->sm_count + B - 1) / B));  // about one wave over the batch
+    PB_TC_DIM_SWITCH(ix->dim, {
+        CKS(set_smem(k_pair_exact<DIM>, smp));
+        k_pair_exact<DIM><<<dim3(pe_ctas, B), 256, smp, ws.stream>>>(
+            ws.xpairs.as<u64>(), ws.xnpairs.as<int>(), pair_cap, ws.Q.as<float>(), ws.qoff.as<int>(), QS,
+            ix->centroids.as<float>(), ix->w_rev.as<float>(), ix->nbits, ix->codes.as<uint32_t>(),
+            ix->residuals.as<uint8_t>(), Mcap, ws.maxkey.as<uint32_t>());
+    });
+    CK(cudaGetLastError());
+    g_stats.launches[PB_STAGE_EXACT] += 5;
+    CKS(launch_exact(ix, ws, ps.kv, B, QS, Mcap, 0, max_tokens, &g_stats.launches[PB_STAGE_EXACT], ws.needexact.as<int>(),
+                     false));
+    KEV_END(PB_KERNEL_EXACT);
+    return PB_OK;
+}
+
+// ---- a7 + a8 exact: only the top_k need exact scores, so the certified tensor-core filter drops the kept docs that
+// provably cannot reach them; the exact MaxSim of the rest, by pairs or by k_exact ----
+static pb_status stage_exact(pb_index *ix, Workspace &ws, const CallPlan &plan, Pass &ps) {
+    const int B = ps.B, QS = ps.QS, Mcap = plan.Mcap;
+    const long long max_tokens = (long long)Mcap * std::max(ix->max_doclen, 1);
+    int *L = g_stats.launches;
+    CKS(ws.maxkey.ensure((size_t)B * Mcap * QS * 4));
+    CKS(ws.exact.ensure((size_t)B * Mcap * 4));
+    CKS(ws.fkeys.ensure((size_t)B * Mcap * 8));
+    // the linear form needs the 16-bit score table of this pass (a flagged query publishes no estimate and keeps
+    // every doc); without a table (PB_FAST_APPROX=0) the decompressing form estimates from fp16 centroids
+    const bool linear = plan.fast && !ix->filter_v1 && ix->tok_inv_norm.p;
+    const float eps_unit = linear ? filter_eps_unit2(ix, ps.tc ? ix->k1_margin : 0) : filter_eps_unit(ix);
+    ps.filt = ix->fast_exact && !plan.io->trace && ix->centroids_f16.p && eps_unit > 0.0f && ps.nq_max <= 64 &&
+              plan.top_k < Mcap && ix->packed % 4 == 0;
+    if (ps.filt) {
+        CKS(ws.est.ensure((size_t)B * Mcap * 4));
+        CKS(ws.kept2.ensure((size_t)B * Mcap * 4));
+        CKS(ws.krank2.ensure((size_t)B * Mcap * 4));
+        CKS(ws.nkept2.ensure((size_t)B * 4 + 16));
+        CKS(ws.tokp2.ensure((size_t)B * (Mcap + 1) * 8));
+        CKS(ws.ktok2.ensure((size_t)B * 8 + 16));
+        if (!plan.fast) {  // the two-pass mode computed it with the score range
+            CKS(ws.qnmax.ensure((size_t)B * 4 + 16));
+            k_query_range<<<B, 256, 0, ws.stream>>>(ws.Q.as<float>(), ws.qoff.as<int>(), ix->dim, ix->cmax, nullptr, nullptr,
+                                                    nullptr, ws.qnmax.as<float>());
+            CK(cudaGetLastError());
+            L[PB_STAGE_EXACT] += 1;
         }
-        if (pairs) {
-            const int pair_cap = 16 * Mcap + 4096;  // ~ (top_k + ties) * nq * (1 + a few) pairs per query in practice
-            CKS(ws.xpairs.ensure((size_t)B * pair_cap * 8));
-            CKS(ws.xnpairs.ensure((size_t)B * 4 + 16));
-            CKS(ws.needexact.ensure((size_t)B * 4 + 16));
-            CK(cudaMemsetAsync(ws.xnpairs.p, 0, (size_t)B * 4, ws.stream));
-            KEV_BEGIN(PB_KERNEL_EXACT);  // pass 2 + pair evaluation + the (normally empty) k_exact of flagged queries
-            CKS(launch_maxsim_tc(ix, ws, kv, B, QS, Mcap, (long long)Mcap * std::max(ix->max_doclen, 1), nq_max,
-                                 ws.estkey.as<uint32_t>(), ws.srcrank.as<uint32_t>(), eps_unit, ws.xpairs.as<u64>(),
-                                 ws.xnpairs.as<int>(), pair_cap, -1));
-            k_pair_overflow<<<(B + 255) / 256, 256, 0, ws.stream>>>(ws.xnpairs.as<int>(), pair_cap, ws.qflag.as<int>(), B,
-                                                                    ws.needexact.as<int>());
-            CK(cudaGetLastError());
-            const size_t smp = ((size_t)(nq_max + 256) * (ix->dim + 1) + 256) * 4;
-            const int pe_ctas = std::max(1, std::min(16, (2 * ix->sm_count + B - 1) / B));  // about one wave over the batch
-            switch (ix->dim) {
-#define PB_PE(DV)                                                                                                      \
-    case DV: {                                                                                                         \
-        CKS(set_smem(k_pair_exact<DV>, smp));                                                                          \
-        k_pair_exact<DV><<<dim3(pe_ctas, B), 256, smp, ws.stream>>>(                                                   \
-            ws.xpairs.as<u64>(), ws.xnpairs.as<int>(), pair_cap, ws.Q.as<float>(), ws.qoff.as<int>(), QS,              \
-            ix->centroids.as<float>(), ix->w_rev.as<float>(), ix->nbits, ix->codes.as<uint32_t>(),                     \
-            ix->residuals.as<uint8_t>(), Mcap, ws.maxkey.as<uint32_t>());                                              \
-    } break;
-                PB_PE(64) PB_PE(96) PB_PE(128)
-#undef PB_PE
-                default: return pb_fail(PB_ERR_UNSUPPORTED, "pair exact: unsupported dim");
+        KeptView kv2{ws.kept2.as<uint32_t>(), ws.nkept2.as<int>(), ws.tokp2.as<long long>(), ws.krank2.as<uint32_t>()};
+        ps.pairs = linear && ix->pair_exact && Mcap <= 65535 && QS <= 256;
+        if (ps.pairs) {
+            CKS(ws.estkey.ensure((size_t)B * Mcap * QS * 4));
+            CKS(ws.srcrank.ensure((size_t)B * Mcap * 4));
+        }
+        CKS(launch_filter(ix, ws, ps.kv, kv2, B, QS, Mcap, plan.top_k, max_tokens, eps_unit, ps.nq_max, linear, ps.pairs,
+                          &L[PB_STAGE_EXACT]));
+        ps.kv = kv2;
+        if (!plan.sharded) ps.kv.krank = nullptr;  // survivors keep their order, so position breaks ties the same way
+    }
+    if (ps.pairs) CKS(launch_pair_exact(ix, ws, plan, ps, eps_unit));
+    else CKS(launch_exact(ix, ws, ps.kv, B, QS, Mcap, 0, max_tokens, &L[PB_STAGE_EXACT]));
+    if (plan.sharded) {
+        CKS(ws.payload.ensure((size_t)B * Mcap * 8));
+        CK(cudaMemsetAsync(ws.fkeys.p, 0xff, (size_t)B * Mcap * 8, ws.stream));  // ~0 = no entry
+    }
+    k_exact_finalize<<<dim3((Mcap + 7) / 8, B), 256, 0, ws.stream>>>(
+        ws.maxkey.as<uint32_t>(), ws.qoff.as<int>(), QS, ps.kv.nkept, Mcap, 0, ws.exact.as<float>(), ws.fkeys.as<u64>(),
+        ps.kv.krank, ps.kv.kept, (uint32_t)ix->doc_id_base, plan.sharded ? ws.payload.as<u64>() : nullptr);
+    CK(cudaGetLastError());
+    L[PB_STAGE_EXACT] += 1;
+    return PB_OK;
+}
+
+// ---- a9 top-k: into the caller's device arrays at the sub-batch's offset, or into staging for the readback;
+// sharded, exchange 2 merges every shard's exact scores ----
+static pb_status stage_topk(pb_index *ix, Workspace &ws, const CallPlan &plan, Pass &ps) {
+    const SearchIO &io = *plan.io;
+    const int B = ps.B, M = plan.M, Mcap = plan.Mcap, top_k = plan.top_k;
+    const int Pm = pow2_ceil(Mcap);
+    if (io.out_on_device) {
+        ps.d_ids = reinterpret_cast<long long *>(io.out_ids) + (size_t)ps.b0 * top_k;
+        ps.d_sc = io.out_scores + (size_t)ps.b0 * top_k;
+        ps.d_cn = io.out_counts + ps.b0;
+    } else {
+        CKS(ws.oids.ensure((size_t)B * top_k * 8));
+        CKS(ws.oscores.ensure((size_t)B * top_k * 4));
+        CKS(ws.ocounts.ensure((size_t)B * 4 + 16));
+        ps.d_ids = ws.oids.as<long long>();
+        ps.d_sc = ws.oscores.as<float>();
+        ps.d_cn = ws.ocounts.as<int>();
+    }
+    if (plan.sharded) {
+        // exchange 2: (exact key | global approx rank) + (doc id | score) of every shard, merged on every rank
+        const int G = ix->world;
+        CKS(ws.gfkeys.ensure((size_t)G * B * M * 8));
+        CKS(ws.gpayload.ensure((size_t)G * B * M * 8));
+        CKS(shard_allgather(ix, ws.stream, ws.fkeys.p, ws.gfkeys.p, (size_t)B * M));
+        CKS(shard_allgather(ix, ws.stream, ws.payload.p, ws.gpayload.p, (size_t)B * M));
+        CKS(ws.mslot.ensure((size_t)B * Mcap * 4));
+        CKS(set_smem(k_merge_topk, (size_t)Pm * 8));
+        k_merge_topk<<<B, 1024, (size_t)Pm * 8, ws.stream>>>(ws.gfkeys.as<u64>(), ws.gpayload.as<u64>(), G, B, M, top_k,
+                                                            ws.mslot.as<uint32_t>(), ps.d_ids, ps.d_sc, ps.d_cn);
+        CK(cudaGetLastError());
+        g_stats.launches[PB_STAGE_TOPK] += 3;
+    } else {
+        CKS(set_smem(k_topk, (size_t)Pm * 8));
+        k_topk<<<B, 1024, (size_t)Pm * 8, ws.stream>>>(ws.fkeys.as<u64>(), ws.exact.as<float>(), ps.kv.kept, ps.kv.nkept, Mcap,
+                                                       top_k, ix->doc_id_base, ps.d_ids, ps.d_sc, ps.d_cn);
+        CK(cudaGetLastError());
+        g_stats.launches[PB_STAGE_TOPK] += 1;
+    }
+    return PB_OK;
+}
+
+// ---- D2H: the pass's counts and flags into ps.host and, for host outputs, the results into ws.hres ----
+static pb_status stage_readback(Workspace &ws, const CallPlan &plan, Pass &ps) {
+    const int B = ps.B, top_k = plan.top_k;
+    const PassHost &h = ps.host;
+    *h.fell = 0;
+    CK(cudaMemcpyAsync(h.n_cells, ws.ncells.p, (size_t)B * 4, cudaMemcpyDeviceToHost, ws.stream));
+    CK(cudaMemcpyAsync(h.n_cand, ws.ncand.p, (size_t)B * 4, cudaMemcpyDeviceToHost, ws.stream));
+    CK(cudaMemcpyAsync(h.n_kept, ws.nkept.p, (size_t)B * 4, cudaMemcpyDeviceToHost, ws.stream));
+    CK(cudaMemcpyAsync(h.counters, ws.counters.p, (size_t)(B + 2) * 8, cudaMemcpyDeviceToHost, ws.stream));
+    if (ps.filt) {
+        CK(cudaMemcpyAsync(h.surv_tokens, ws.ktok2.p, (size_t)B * 8, cudaMemcpyDeviceToHost, ws.stream));
+        CK(cudaMemcpyAsync(h.survivors, ws.nkept2.p, (size_t)B * 4, cudaMemcpyDeviceToHost, ws.stream));
+    }
+    if (plan.fast) CK(cudaMemcpyAsync(h.rechecked, ws.ncand2.p, (size_t)B * 4, cudaMemcpyDeviceToHost, ws.stream));
+    if (ps.pairs) {
+        CK(cudaMemcpyAsync(h.pairs, ws.xnpairs.p, (size_t)B * 4, cudaMemcpyDeviceToHost, ws.stream));
+        CK(cudaMemcpyAsync(h.need_exact, ws.needexact.p, (size_t)B * 4, cudaMemcpyDeviceToHost, ws.stream));
+    }
+    if (ps.d_fallback) CK(cudaMemcpyAsync(h.fell, ps.d_fallback, 4, cudaMemcpyDeviceToHost, ws.stream));
+    if (!plan.io->out_on_device) {
+        CKS(ws.hres.ensure((size_t)B * top_k * 12 + (size_t)B * 4));
+        char *r = ws.hres.as<char>();
+        CK(cudaMemcpyAsync(r, ps.d_ids, (size_t)B * top_k * 8, cudaMemcpyDeviceToHost, ws.stream));
+        CK(cudaMemcpyAsync(r + (size_t)B * top_k * 8, ps.d_sc, (size_t)B * top_k * 4, cudaMemcpyDeviceToHost, ws.stream));
+        CK(cudaMemcpyAsync(r + (size_t)B * top_k * 12, ps.d_cn, (size_t)B * 4, cudaMemcpyDeviceToHost, ws.stream));
+    }
+    return PB_OK;
+}
+
+// ---- the pass's stage and kernel times (profiling) and its work counters, from what the readback brought ----
+static pb_status stage_accounting(pb_index *ix, Workspace &ws, const CallPlan &plan, const Pass &ps) {
+    const int B = ps.B;
+    const PassHost &h = ps.host;
+    pb_work_counters &w = g_stats.work;
+    if (ix->profiling) {
+        for (int s = 0; s < PB_STAGE_COUNT; ++s) {
+            float ms = 0.f;
+            CK(cudaEventElapsedTime(&ms, ws.ev[s], ws.ev[s + 1]));
+            g_stats.ms[s] += ms;
+        }
+        for (int k = 0; k < PB_KERNEL_COUNT; ++k)
+            if (g_stats.kernel_seen[k]) {
+                float ms = 0.f;
+                CK(cudaEventElapsedTime(&ms, ws.kev[2 * k], ws.kev[2 * k + 1]));
+                g_stats.kernel_ms[k] += ms;
+                g_stats.kernel_seen[k] = false;
             }
-            CK(cudaGetLastError());
-            L[PB_STAGE_EXACT] += 5;
-            CKS(launch_exact(ix, ws, kv, B, QS, Mcap, 0, (long long)Mcap * std::max(ix->max_doclen, 1), &L[PB_STAGE_EXACT],
-                             ws.needexact.as<int>(), false));
-            KEV_END(PB_KERNEL_EXACT);
+    }
+    if (plan.fast && ix->k1_diag && ws.k1diag.p) {
+        int got[2] = {0, 0};
+        CK(cudaMemcpy(got, ws.k1diag.p, 8, cudaMemcpyDeviceToHost));
+        w.k1_tc_max_code_diff = std::max<long long>(w.k1_tc_max_code_diff, got[0]);
+    }
+    w.n_queries += B;
+    w.n_query_tokens += ps.R;
+    switch (ps.probe) {
+        case ProbeMode::TensorCore: w.n_k1_tc += 1; break;
+        case ProbeMode::Threshold: (*h.fell ? w.n_probe_list : w.n_probe_threshold) += 1; break;
+        case ProbeMode::List: w.n_probe_list += 1; break;
+        case ProbeMode::AllEligible:
+        case ProbeMode::BigProbe: break;
+    }
+    if (plan.fast)
+        for (int b = 0; b < B; ++b) w.n_recheck_docs += h.rechecked[b];
+    if (ps.pairs)
+        for (int b = 0; b < B; ++b) {
+            if (h.need_exact[b]) w.n_pair_fallback_queries += 1;
+            else w.n_exact_pairs += h.pairs[b];
+        }
+    w.n_candidate_tokens += (long long)h.counters[0];
+    for (int b = 0; b < B; ++b) {
+        w.n_cells += h.n_cells[b];
+        w.n_candidates += h.n_cand[b];
+        if (ps.filt) {
+            w.n_filter_docs += h.n_kept[b];
+            w.n_filter_tokens += (long long)h.counters[1 + b];
+            w.n_exact_docs += h.survivors[b];
+            w.n_exact_tokens += h.surv_tokens[b];
         } else {
-            CKS(launch_exact(ix, ws, kv, B, QS, Mcap, 0, (long long)Mcap * std::max(ix->max_doclen, 1), &L[PB_STAGE_EXACT]));
+            w.n_exact_docs += h.n_kept[b];
+            w.n_exact_tokens += (long long)h.counters[1 + b];
         }
-        if (sharded) {
-            CKS(ws.payload.ensure((size_t)B * Mcap * 8));
-            CK(cudaMemsetAsync(ws.fkeys.p, 0xff, (size_t)B * Mcap * 8, ws.stream));  // ~0 = no entry
-        }
-        k_exact_finalize<<<dim3((Mcap + 7) / 8, B), 256, 0, ws.stream>>>(
-            ws.maxkey.as<uint32_t>(), ws.qoff.as<int>(), QS, kv.nkept, Mcap, 0, ws.exact.as<float>(),
-            ws.fkeys.as<u64>(), kv.krank, kv.kept, (uint32_t)ix->doc_id_base, sharded ? ws.payload.as<u64>() : nullptr);
-        CK(cudaGetLastError());
-        L[PB_STAGE_EXACT] += 1;
-        if (prof) CK(cudaEventRecord(ws.ev[7], ws.stream));
+    }
+    return PB_OK;
+}
 
-        // ---- a9 top-k ----
-        long long *d_ids;
-        float *d_sc;
-        int *d_cn;
-        if (io.out_on_device) {
-            d_ids = reinterpret_cast<long long *>(io.out_ids) + (size_t)b0 * top_k;
-            d_sc = io.out_scores + (size_t)b0 * top_k;
-            d_cn = io.out_counts + b0;
-        } else {
-            CKS(ws.oids.ensure((size_t)B * top_k * 8));
-            CKS(ws.oscores.ensure((size_t)B * top_k * 4));
-            CKS(ws.ocounts.ensure((size_t)B * 4 + 16));
-            d_ids = ws.oids.as<long long>();
-            d_sc = ws.oscores.as<float>();
-            d_cn = ws.ocounts.as<int>();
+// ---- the trace of a pass (tests only; synchronous copies) ----
+static pb_status stage_trace(pb_index *ix, Workspace &ws, const CallPlan &plan, const Pass &ps) {
+    pb_trace *t = plan.io->trace;
+    if (!t) return PB_OK;
+    const PassHost &h = ps.host;
+    for (int b = 0; b < ps.B; ++b) {
+        const int64_t gb = ps.b0 + b;
+        if (t->n_cells) t->n_cells[gb] = h.n_cells[b];
+        if (t->n_candidates) t->n_candidates[gb] = h.n_cand[b];
+        if (t->n_kept) t->n_kept[gb] = h.n_kept[b];
+        if (t->cells) {
+            int n = (int)std::min<int64_t>(h.n_cells[b], t->cells_cap);
+            std::vector<uint32_t> tmp(n);
+            CK(cudaMemcpy(tmp.data(), ws.cells.as<uint32_t>() + (size_t)b * ps.cells_cap, (size_t)n * 4, cudaMemcpyDeviceToHost));
+            for (int i = 0; i < n; ++i) t->cells[gb * t->cells_cap + i] = tmp[i];
         }
-        if (sharded) {
-            // exchange 2: (exact key | global approx rank) + (doc id | score) of every shard, merged on every rank
-            const int G = ix->world;
-            CKS(ws.gfkeys.ensure((size_t)G * B * M * 8));
-            CKS(ws.gpayload.ensure((size_t)G * B * M * 8));
-            CKS(shard_allgather(ix, ws.stream, ws.fkeys.p, ws.gfkeys.p, (size_t)B * M));
-            CKS(shard_allgather(ix, ws.stream, ws.payload.p, ws.gpayload.p, (size_t)B * M));
-            CKS(ws.mslot.ensure((size_t)B * Mcap * 4));
-            CKS(set_smem(k_merge_topk, (size_t)Pm * 8));
-            k_merge_topk<<<B, 1024, (size_t)Pm * 8, ws.stream>>>(ws.gfkeys.as<u64>(), ws.gpayload.as<u64>(), G, B, M, top_k,
-                                                                ws.mslot.as<uint32_t>(), d_ids, d_sc, d_cn);
-            CK(cudaGetLastError());
-            L[PB_STAGE_TOPK] += 3;
-        } else {
-            CKS(set_smem(k_topk, (size_t)Pm * 8));
-            k_topk<<<B, 1024, (size_t)Pm * 8, ws.stream>>>(ws.fkeys.as<u64>(), ws.exact.as<float>(), kv.kept, kv.nkept, Mcap,
-                                                           top_k, ix->doc_id_base, d_ids, d_sc, d_cn);
-            CK(cudaGetLastError());
-            L[PB_STAGE_TOPK] += 1;
+        if (t->candidates || t->approx) {
+            int n = (int)std::min<int64_t>(h.n_cand[b], t->cand_cap);
+            std::vector<uint32_t> tmp(n);
+            CK(cudaMemcpy(tmp.data(), ws.cand.as<uint32_t>() + (size_t)b * ix->D, (size_t)n * 4, cudaMemcpyDeviceToHost));
+            if (t->candidates)
+                for (int i = 0; i < n; ++i) t->candidates[gb * t->cand_cap + i] = (int64_t)tmp[i] + ix->doc_id_base;
+            if (t->approx)
+                CK(cudaMemcpy(t->approx + gb * t->cand_cap, ws.approx.as<float>() + (size_t)b * ix->D, (size_t)n * 4,
+                              cudaMemcpyDeviceToHost));
         }
-        if (prof) CK(cudaEventRecord(ws.ev[8], ws.stream));
+        if (t->kept || t->kept_exact) {
+            int n = (int)std::min<int64_t>(h.n_kept[b], t->kept_cap);
+            std::vector<uint32_t> tmp(n);
+            CK(cudaMemcpy(tmp.data(), ws.kept.as<uint32_t>() + (size_t)b * plan.Mcap, (size_t)n * 4, cudaMemcpyDeviceToHost));
+            if (t->kept)
+                for (int i = 0; i < n; ++i) t->kept[gb * t->kept_cap + i] = (int64_t)tmp[i] + ix->doc_id_base;
+            if (t->kept_exact)
+                CK(cudaMemcpy(t->kept_exact + gb * t->kept_cap, ws.exact.as<float>() + (size_t)b * plan.Mcap, (size_t)n * 4,
+                              cudaMemcpyDeviceToHost));
+        }
+    }
+    return PB_OK;
+}
 
-        // ---- D2H ----
-        // pinned layout after the (B + 1) query offsets: u64 counters[B + 2] | i64 survivor tokens[B] |
-        // int n_cells[B], n_cand[B], n_kept[B], survivors[B], re-checked[B], probe fallback flag
-        char *hbase = ws.hcounts.as<char>() + (((size_t)(B + 1) * 4 + 15) & ~(size_t)15);
-        unsigned long long *hcnt = reinterpret_cast<unsigned long long *>(hbase);
-        long long *hsurv_tok = reinterpret_cast<long long *>(hcnt + (B + 2));
-        int *hc = reinterpret_cast<int *>(hsurv_tok + B);
-        int *hsurv = hc + 3 * B, *hrecheck = hc + 4 * B, *hfell = hc + 5 * B, *hpairs = hc + 5 * B + 16, *hneed = hc + 6 * B + 16;
-        *hfell = 0;
-        CK(cudaMemcpyAsync(hc, ws.ncells.p, (size_t)B * 4, cudaMemcpyDeviceToHost, ws.stream));
-        CK(cudaMemcpyAsync(hc + B, ws.ncand.p, (size_t)B * 4, cudaMemcpyDeviceToHost, ws.stream));
-        CK(cudaMemcpyAsync(hc + 2 * B, ws.nkept.p, (size_t)B * 4, cudaMemcpyDeviceToHost, ws.stream));
-        CK(cudaMemcpyAsync(hcnt, ws.counters.p, (size_t)(B + 2) * 8, cudaMemcpyDeviceToHost, ws.stream));
-        if (filt) {
-            CK(cudaMemcpyAsync(hsurv_tok, ws.ktok2.p, (size_t)B * 8, cudaMemcpyDeviceToHost, ws.stream));
-            CK(cudaMemcpyAsync(hsurv, ws.nkept2.p, (size_t)B * 4, cudaMemcpyDeviceToHost, ws.stream));
-        }
-        if (fast) CK(cudaMemcpyAsync(hrecheck, ws.ncand2.p, (size_t)B * 4, cudaMemcpyDeviceToHost, ws.stream));
-        if (pairs) {
-            CK(cudaMemcpyAsync(hpairs, ws.xnpairs.p, (size_t)B * 4, cudaMemcpyDeviceToHost, ws.stream));
-            CK(cudaMemcpyAsync(hneed, ws.needexact.p, (size_t)B * 4, cudaMemcpyDeviceToHost, ws.stream));
-        }
-        if (d_probe_fallback) CK(cudaMemcpyAsync(hfell, d_probe_fallback, 4, cudaMemcpyDeviceToHost, ws.stream));
-        if (!io.out_on_device) {
-            size_t bytes = (size_t)B * top_k * 12 + (size_t)B * 4;
-            CKS(ws.hres.ensure(bytes));
-            char *h = ws.hres.as<char>();
-            CK(cudaMemcpyAsync(h, d_ids, (size_t)B * top_k * 8, cudaMemcpyDeviceToHost, ws.stream));
-            CK(cudaMemcpyAsync(h + (size_t)B * top_k * 8, d_sc, (size_t)B * top_k * 4, cudaMemcpyDeviceToHost, ws.stream));
-            CK(cudaMemcpyAsync(h + (size_t)B * top_k * 12, d_cn, (size_t)B * 4, cudaMemcpyDeviceToHost, ws.stream));
-        }
-        if (prof) CK(cudaEventRecord(ws.ev[9], ws.stream));
-        CK(cudaStreamSynchronize(ws.stream));
-        if (tc && *hfell) {  // the tensor-core pass gave up on the device: same sub-batch again on the exact path
+// One pass over the sub-batch at b0, stage by stage, with the stage events ws.ev[0..9] between them.  The first pass
+// takes the tensor-core path where the call and the sub-batch's rows allow it: a flagged query, a probe-list overflow or
+// a re-check overflow raises a device flag instead of being read back mid-way; the pass then finishes on (memory-safe)
+// garbage and *redo asks for a second pass, on the exact path.  On a sharded handle every rank votes on its first pass,
+// whatever path it takes: the ranks' flags are gathered before the first exchange, so that every rank abandons the
+// pass together and the ranks' exchanges stay paired.
+static pb_status run_pass(pb_index *ix, Workspace &ws, const CallPlan &plan, int64_t b0, bool first, bool *redo) {
+    auto mark = [&](int s) -> pb_status {
+        if (ix->profiling) CK(cudaEventRecord(ws.ev[s], ws.stream));
+        return PB_OK;
+    };
+    *redo = false;
+    Pass ps;
+    ps.b0 = b0;
+    CKS(mark(0));
+    CKS(stage_h2d(ix, ws, plan, ps));
+    CKS(mark(1));
+    ps.tc = first && plan.tc_call && ps.QS / 8 <= 32;
+    ps.probe = probe_mode(ix, plan, ps.QS, ps.tc);
+    CKS(stage_scores(ix, ws, plan, ps));
+    CKS(mark(2));
+    CKS(stage_probe(ix, ws, plan, ps));
+    CKS(mark(3));
+    CKS(stage_candidates(ix, ws, plan, ps));
+    CKS(mark(4));
+    CKS(stage_approx(ix, ws, plan, ps));
+    CKS(mark(5));
+    if (first && plan.sharded) {
+        // The probe flags are the same on every rank (a2/a3 are replicated), a re-check overflow is not: it depends
+        // on this shard's documents.  Nor is the path: a rank without tensor-core operands (a shard with no tokens)
+        // or with other settings runs the exact pass and votes 0.  Every rank's flag word is gathered here, before
+        // exchange 1, and the pass is abandoned on all ranks if any rank raised it; a lone redo would pair its
+        // exchanges with the peers' next ones.  The kernels so far have restored their scratch invariants
+        // (bitmaps, re-check maxima).
+        const u64 *all = nullptr;
+        CKS(shard_vote(ix, ws, 0, ps.tc ? ps.d_fallback : nullptr, &all));
+        u64 any = 0;
+        for (int g = 0; g < ix->world; ++g) any |= all[g];
+        if (any) {
             *redo = true;
             return PB_OK;
         }
-        if (!io.out_on_device) {
-            char *h = ws.hres.as<char>();
-            memcpy(io.out_ids + (size_t)b0 * top_k, h, (size_t)B * top_k * 8);
-            memcpy(io.out_scores + (size_t)b0 * top_k, h + (size_t)B * top_k * 8, (size_t)B * top_k * 4);
-            memcpy(io.out_counts + b0, h + (size_t)B * top_k * 12, (size_t)B * 4);
-        }
-        if (prof) {
-            for (int s = 0; s < PB_STAGE_COUNT; ++s) {
-                float ms = 0.f;
-                CK(cudaEventElapsedTime(&ms, ws.ev[s], ws.ev[s + 1]));
-                g_stats.ms[s] += ms;
-            }
-            for (int k = 0; k < PB_KERNEL_COUNT; ++k)
-                if (g_stats.kernel_seen[k]) {
-                    float ms = 0.f;
-                    CK(cudaEventElapsedTime(&ms, ws.kev[2 * k], ws.kev[2 * k + 1]));
-                    g_stats.kernel_ms[k] += ms;
-                    g_stats.kernel_seen[k] = false;
-                }
-        }
-        if (fast && ix->k1_diag && ws.k1diag.p) {
-            int got[2] = {0, 0};
-            CK(cudaMemcpy(got, ws.k1diag.p, 8, cudaMemcpyDeviceToHost));
-            g_stats.work.k1_tc_max_code_diff = std::max<long long>(g_stats.work.k1_tc_max_code_diff, got[0]);
-            g_stats.work.k1_rows_mismatch += 0;
-        }
-        g_stats.work.n_queries += B;
-        g_stats.work.n_query_tokens += R;
-        if (tc) g_stats.work.n_k1_tc += 1;
-        else if (d_probe_fallback) (*hfell ? g_stats.work.n_probe_list : g_stats.work.n_probe_threshold) += 1;
-        else if (probe_list_only) g_stats.work.n_probe_list += 1;
-        if (fast)
-            for (int b = 0; b < B; ++b) g_stats.work.n_recheck_docs += hrecheck[b];
-        if (pairs)
-            for (int b = 0; b < B; ++b) {
-                if (hneed[b]) g_stats.work.n_pair_fallback_queries += 1;
-                else g_stats.work.n_exact_pairs += hpairs[b];
-            }
-        g_stats.work.n_candidate_tokens += (long long)hcnt[0];
-        for (int b = 0; b < B; ++b) {
-            g_stats.work.n_cells += hc[b];
-            g_stats.work.n_candidates += hc[B + b];
-            if (filt) {
-                g_stats.work.n_filter_docs += hc[2 * B + b];
-                g_stats.work.n_filter_tokens += (long long)hcnt[1 + b];
-                g_stats.work.n_exact_docs += hsurv[b];
-                g_stats.work.n_exact_tokens += hsurv_tok[b];
-            } else {
-                g_stats.work.n_exact_docs += hc[2 * B + b];
-                g_stats.work.n_exact_tokens += (long long)hcnt[1 + b];
-            }
-        }
-        // ---- optional trace (tests only; synchronous copies) ----
-        if (io.trace) {
-            pb_trace *t = io.trace;
-            for (int b = 0; b < B; ++b) {
-                const int64_t gb = b0 + b;
-                if (t->n_cells) t->n_cells[gb] = hc[b];
-                if (t->n_candidates) t->n_candidates[gb] = hc[B + b];
-                if (t->n_kept) t->n_kept[gb] = hc[2 * B + b];
-                if (t->cells) {
-                    int n = (int)std::min<int64_t>(hc[b], t->cells_cap);
-                    std::vector<uint32_t> tmp(n);
-                    CK(cudaMemcpy(tmp.data(), ws.cells.as<uint32_t>() + (size_t)b * cells_cap, (size_t)n * 4, cudaMemcpyDeviceToHost));
-                    for (int i = 0; i < n; ++i) t->cells[gb * t->cells_cap + i] = tmp[i];
-                }
-                if (t->candidates || t->approx) {
-                    int n = (int)std::min<int64_t>(hc[B + b], t->cand_cap);
-                    std::vector<uint32_t> tmp(n);
-                    CK(cudaMemcpy(tmp.data(), ws.cand.as<uint32_t>() + (size_t)b * ix->D, (size_t)n * 4, cudaMemcpyDeviceToHost));
-                    if (t->candidates)
-                        for (int i = 0; i < n; ++i) t->candidates[gb * t->cand_cap + i] = (int64_t)tmp[i] + ix->doc_id_base;
-                    if (t->approx)
-                        CK(cudaMemcpy(t->approx + gb * t->cand_cap, ws.approx.as<float>() + (size_t)b * ix->D, (size_t)n * 4,
-                                      cudaMemcpyDeviceToHost));
-                }
-                if (t->kept || t->kept_exact) {
-                    int n = (int)std::min<int64_t>(hc[2 * B + b], t->kept_cap);
-                    std::vector<uint32_t> tmp(n);
-                    CK(cudaMemcpy(tmp.data(), ws.kept.as<uint32_t>() + (size_t)b * Mcap, (size_t)n * 4, cudaMemcpyDeviceToHost));
-                    if (t->kept)
-                        for (int i = 0; i < n; ++i) t->kept[gb * t->kept_cap + i] = (int64_t)tmp[i] + ix->doc_id_base;
-                    if (t->kept_exact)
-                        CK(cudaMemcpy(t->kept_exact + gb * t->kept_cap, ws.exact.as<float>() + (size_t)b * Mcap, (size_t)n * 4,
-                                      cudaMemcpyDeviceToHost));
-                }
-            }
-        }
+    }
+    CKS(stage_cut(ix, ws, plan, ps));
+    CKS(mark(6));
+    CKS(stage_exact(ix, ws, plan, ps));
+    CKS(mark(7));
+    CKS(stage_topk(ix, ws, plan, ps));
+    CKS(mark(8));
+    CKS(stage_readback(ws, plan, ps));
+    CKS(mark(9));
+    CK(cudaStreamSynchronize(ws.stream));
+    if (ps.tc && *ps.host.fell) {  // the tensor-core pass gave up on the device: same sub-batch again on the exact path
+        *redo = true;
         return PB_OK;
-        };  // run_sub
+    }
+    const SearchIO &io = *plan.io;
+    if (!io.out_on_device) {
+        const size_t n = (size_t)ps.B * plan.top_k;
+        const char *r = ws.hres.as<char>();
+        memcpy(io.out_ids + (size_t)ps.b0 * plan.top_k, r, n * 8);
+        memcpy(io.out_scores + (size_t)ps.b0 * plan.top_k, r + n * 8, n * 4);
+        memcpy(io.out_counts + ps.b0, r + n * 12, (size_t)ps.B * 4);
+    }
+    CKS(stage_accounting(ix, ws, plan, ps));
+    return stage_trace(ix, ws, plan, ps);
+}
+
+// `lanes`: how many slices of the caller's batch run concurrently (search_impl); they share the workspace budget
+static pb_status search_impl_inner(pb_index *ix, const pb_search_params *p, const SearchIO &io, int lanes) {
+    WorkspaceLease lease{ix};
+    CallPlan plan;
+    CKS(plan_call(ix, p, io, lanes, lease, plan));
+    if (plan.Bt == 0) return PB_OK;
+    Workspace &ws = *lease.ws;
+    if (plan.empty) {
+        if (io.out_on_device) CK(cudaMemsetAsync(io.out_counts, 0, (size_t)plan.Bt * 4, ws.stream));
+        else memset(io.out_counts, 0, (size_t)plan.Bt * 4);
+        CK(cudaStreamSynchronize(ws.stream));
+        lease.done = true;
+        return PB_OK;
+    }
+    const bool prof = ix->profiling;
+    if (prof) CK(cudaEventRecord(ws.call_ev[0], ws.stream));
+    for (int64_t b0 = 0; b0 < plan.Bt; b0 += plan.QB) {
         bool redo = false;
-        CKS(run_sub(want_tc, sharded, &redo));
+        CKS(run_pass(ix, ws, plan, b0, true, &redo));
         if (redo) {
             g_stats.work.n_k1_tc_redo += 1;
-            CKS(run_sub(false, false, &redo));
+            CKS(run_pass(ix, ws, plan, b0, false, &redo));
         }
     }
     if (prof) {
@@ -1895,7 +2022,7 @@ static pb_status search_impl_inner(pb_index *ix, const pb_search_params *p, cons
         CK(cudaEventSynchronize(ws.call_ev[1]));
         CK(cudaEventElapsedTime(&g_stats.call_ms, ws.call_ev[0], ws.call_ev[1]));
     }
-    rel.ok = true;
+    lease.done = true;
     return PB_OK;
 }
 
@@ -1932,7 +2059,7 @@ static pb_status search_impl(pb_index *ix, const pb_search_params *p, const Sear
         if (!lane_lock.owns_lock()) lanes = 1;  // another host thread is using the helpers: it already provides the overlap
     }
     if (lanes <= 1) {
-        const pb_status st = search_impl_inner(ix, p, io);
+        const pb_status st = search_impl_inner(ix, p, io, 1);
         if (st != PB_OK && ix && ix->group) ix->group->fail();  // the peers must not wait for a rank that gave up
         return st;
     }
@@ -1963,9 +2090,7 @@ static pb_status search_impl(pb_index *ix, const pb_search_params *p, const Sear
         ios[l].out_counts = io.out_counts ? io.out_counts + b0 : nullptr;
     }
     auto run_lane = [&](int l) {
-        g_budget_div = lanes;
-        sts[l] = search_impl_inner(ix, p, ios[l]);
-        g_budget_div = 1;
+        sts[l] = search_impl_inner(ix, p, ios[l], lanes);
         stats[l] = g_stats;
         if (sts[l] != PB_OK) errs[l] = g_err;
     };
@@ -2021,14 +2146,9 @@ extern "C" pb_status pb_centroid_scores(pb_index *ix, const float *query_tokens,
     if (!ix || (!query_tokens && n) || (!out && n)) return pb_fail(PB_ERR_INVALID, "null argument");
     if (n == 0) return PB_OK;
     CK(cudaSetDevice(ix->device));
-    std::unique_ptr<Workspace> wsp;
-    CKS(ix->acquire(wsp));
-    Workspace &ws = *wsp;
-    struct Releaser {
-        pb_index *ix;
-        std::unique_ptr<Workspace> &w;
-        ~Releaser() { ix->release(w); }
-    } rel{ix, wsp};
+    WorkspaceLease lease{ix};
+    CKS(lease.acquire());
+    Workspace &ws = *lease.ws;
     // one pseudo-query per block of <= 64 tokens keeps the per-query transposed layout small
     const int blk = 64;
     DevBuf S;
@@ -2042,12 +2162,13 @@ extern "C" pb_status pb_centroid_scores(pb_index *ix, const float *query_tokens,
         CK(cudaMemcpyAsync(ws.Q.p, query_tokens + (size_t)r0 * ix->dim, (size_t)nq * ix->dim * 4, cudaMemcpyHostToDevice, ws.stream));
         CK(cudaMemcpyAsync(ws.qoff.p, qoff, 8, cudaMemcpyHostToDevice, ws.stream));
         CKS(ws.ST.ensure((size_t)ix->K * QS * 4));
-        CKS(launch_centroid_scores(ix, ws, 1, QS, nullptr));
+        CKS(launch_centroid_scores(ix, ws, 1, QS, nullptr, false));
         k_transpose_scores<<<(unsigned)((ix->K + 255) / 256), 256, 0, ws.stream>>>(ws.ST.as<float>(), ix->K, QS, nq, S.as<float>());
         CK(cudaGetLastError());
         CK(cudaMemcpyAsync(out + (size_t)r0 * ix->K, S.p, (size_t)nq * ix->K * 4, cudaMemcpyDeviceToHost, ws.stream));
         CK(cudaStreamSynchronize(ws.stream));
     }
+    lease.done = true;
     return PB_OK;
 }
 
@@ -2127,19 +2248,13 @@ extern "C" pb_status pb_maxsim_scores(int32_t device, const float *query, int32_
     CKS(dex.ensure((size_t)Mcap * 4));
     long long chunks = (total + PB_TOK_TILE - 1) / PB_TOK_TILE;
     int gx = (int)std::max<long long>(1, std::min<long long>(chunks, 148ll * 16));
-    switch (dim) {
-#define PB_CASE(DV)                                                                                              \
-    case DV: {                                                                                                   \
-        auto kern = k_exact<DV, true>;                                                                           \
-        CKS(set_smem(kern, smem_exact(DV, 0)));                                                                  \
-        kern<<<dim3(gx, 1), 128, smem_exact(DV, 0)>>>(dQ.as<float>(), dqoff.as<int>(), QS, nullptr, nullptr, 8, nullptr, \
-                                                   nullptr, nullptr, dtok.as<float>(), dkept.as<uint32_t>(),    \
-                                                   dnk.as<int>(), dtp.as<long long>(), Mcap, 0, dmax.as<uint32_t>(), nullptr); \
-    } break;
-        PB_CASE(32) PB_CASE(64) PB_CASE(96) PB_CASE(128) PB_CASE(256)
-#undef PB_CASE
-        default: break;
-    }
+    PB_DIM_SWITCH(dim, {
+        auto kern = k_exact<DIM, true>;
+        CKS(set_smem(kern, smem_exact(DIM, 0)));
+        kern<<<dim3(gx, 1), 128, smem_exact(DIM, 0)>>>(dQ.as<float>(), dqoff.as<int>(), QS, nullptr, nullptr, 8, nullptr,
+                                                    nullptr, nullptr, dtok.as<float>(), dkept.as<uint32_t>(),
+                                                    dnk.as<int>(), dtp.as<long long>(), Mcap, 0, dmax.as<uint32_t>(), nullptr);
+    });
     CK(cudaGetLastError());
     k_exact_finalize<<<dim3((Mcap + 7) / 8, 1), 256>>>(dmax.as<uint32_t>(), dqoff.as<int>(), QS, dnk.as<int>(), Mcap, 0,
                                                       dex.as<float>(), nullptr, nullptr, nullptr, 0u, nullptr);
@@ -2153,14 +2268,9 @@ extern "C" pb_status pb_exhaustive_scores(pb_index *ix, const float *queries, co
     if (!ix || (!queries && n_queries) || !q_off || (!out_scores && n_queries)) return pb_fail(PB_ERR_INVALID, "null argument");
     CK(cudaSetDevice(ix->device));
     if (n_queries == 0 || ix->D == 0) return PB_OK;
-    std::unique_ptr<Workspace> wsp;
-    CKS(ix->acquire(wsp));
-    Workspace &ws = *wsp;
-    struct Releaser {
-        pb_index *ix;
-        std::unique_ptr<Workspace> &w;
-        ~Releaser() { ix->release(w); }
-    } rel{ix, wsp};
+    WorkspaceLease lease{ix};
+    CKS(lease.acquire());
+    Workspace &ws = *lease.ws;
     std::vector<long long> doff((size_t)ix->D + 1);
     CK(cudaMemcpy(doff.data(), ix->doc_off.p, doff.size() * 8, cudaMemcpyDeviceToHost));
     const int QBmax = 32;
@@ -2201,6 +2311,7 @@ extern "C" pb_status pb_exhaustive_scores(pb_index *ix, const float *queries, co
             CK(cudaStreamSynchronize(ws.stream));
         }
     }
+    lease.done = true;
     return PB_OK;
 }
 
